@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the B200 CP-CALS hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|4|5]
-                    [--weak] [--no-secondary] [--no-cpu-baseline]
+                    [--weak] [--no-secondary] [--no-cpu-baseline] [--dump-outputs DIR]
 
 Metric (BASELINE.json): concurrent-ALS iterations per second summed over all models ("model-iterations/s").  The
 headline workload is BASELINE config 2 (the largest configuration the metric is quoted on that fits one GPU): synthetic
@@ -23,6 +23,11 @@ reference's own experiments, src/experiments/experiments.cpp:62-63).
              iterations: largest relative error over every factor matrix, lambda and fit of all models
   cpu_baseline : the unmodified reference timed on the box's host cores on a bounded sample
   secondary    : the other BASELINE configurations at the same GPU count, each with its own clocks / roofline / e2e
+
+--dump-outputs DIR writes the fitted models of the last timed step of the headline run as float64 .npy files, so that
+two builds can be compared output for output: the inputs are seeded and identical from run to run.  On N > 1 GPUs only
+rank 0 writes, and what it writes is its own share: the models shard_models assigns to rank 0 (strong scaling), or
+rank 0's own model set (--weak); the sliced config 5 replicates the models, so there it is the whole set.
 
 N > 1 (torchrun): the tensor is replicated and ONE model set (for the jackknife: one set of leave-one-out sub-models) is
 sharded over the ranks -- strong scaling, no collective on the data path (north_star's partition; SURVEY 8e).  `--weak`
@@ -373,6 +378,21 @@ class Dist:
         return self._reduce(x, self.dist.ReduceOp.SUM) if self.dist is not None else x
 
 
+def dump_outputs(eng, out_dir):
+    """The models of the engine's last run as a caller of cp_cals receives them: per mode the factor matrices of all
+    models side by side (I_n x sum of ranks, queue order), lambda, and per model the iteration count, error and fit.
+    Every file is float64; the largest configuration (config 3) comes to about 37 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    res = eng.fetch_all()
+    arrays = {"lambda": np.concatenate([lam for _, lam, _ in res])}
+    for n in range(len(eng.modes)):
+        arrays["factors_mode%d" % n] = np.concatenate([fs[n] for fs, _, _ in res], axis=1)
+    for key in ("iters", "error", "fit"):
+        arrays[key] = np.array([getattr(st, key) for _, _, st in res])
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def cpp_e2e(cfg, X, models, jk, als_iters, steps, warmup, device, no_pair_node=False, nnls=False):
     """The end-to-end leg through the drop-in C++ API: examples/bench_e2e.cpp (cals::cp_cals of libcals.so) on a case
     file holding exactly these inputs.  Returns its JSON dict, or None when the program is missing / failed."""
@@ -396,7 +416,7 @@ def cpp_e2e(cfg, X, models, jk, als_iters, steps, warmup, device, no_pair_node=F
     return None
 
 
-def run_sharded(args, cfg_id, rank, world, local_rank, D, steps, warmup, main_line):
+def run_sharded(args, cfg_id, rank, world, local_rank, D, steps, warmup, main_line, dump_dir=None):
     """Configs 1-4: tensor replicated, model set sharded over the ranks.  Returns the line (rank 0) or None."""
     import importlib
 
@@ -456,6 +476,8 @@ def run_sharded(args, cfg_id, rank, world, local_rank, D, steps, warmup, main_li
     done_w = int(D.max(done_w))
     ev_ms, wall, reps = timed(eng.rerun, steps)
     clocks = sampler.stop()
+    if dump_dir and rank == 0:
+        dump_outputs(eng, dump_dir)
     launches = sum(r.kernel_launches for r in reps)
     assert all(r.iter == als_iters and r.n_ktensors == n_models for r in reps)
     ev_ms = D.max(ev_ms)       # CUDA events on the engine stream around the K steps, max over ranks
@@ -651,7 +673,7 @@ def run_sharded(args, cfg_id, rank, world, local_rank, D, steps, warmup, main_li
     return line
 
 
-def run_sliced(args, cfg_id, rank, world, local_rank, D, steps, warmup):
+def run_sliced(args, cfg_id, rank, world, local_rank, D, steps, warmup, dump_dir=None):
     """BASELINE config 5: ONE tensor sliced over the ranks (strong scaling), all models replicated."""
     import importlib
 
@@ -705,6 +727,8 @@ def run_sliced(args, cfg_id, rank, world, local_rank, D, steps, warmup):
         eng.rerun()
     ev_ms, wall, reps = timed(eng.rerun, steps)
     clocks = sampler.stop()
+    if dump_dir and rank == 0:
+        dump_outputs(eng, dump_dir)
     ev_ms, wall = D.max(ev_ms), D.max(wall)
     value = n_models * als_iters * steps / (ev_ms * 1e-3)
     launches = sum(r.kernel_launches for r in reps)
@@ -789,7 +813,14 @@ def main():
     ap.add_argument("--no-pair-node", action="store_true", help="measurement aid: one full MTTKRP per mode (3-mode "
                     "tensors otherwise share one contraction between modes 1 and 2, csrc/pairnode.cuh)")
     ap.add_argument("--nnls", action="store_true", help="measurement aid: update_method = NNLS instead of the Cholesky solve")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the fitted models of the headline run's "
+                    "last timed step to DIR/<name>.npy (float64) for output-for-output comparison of builds; on N > 1 "
+                    "GPUs, rank 0's share of the model set")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     main_cfg = args.config if args.config is not None else 2
     cfg = CONFIGS[main_cfg]
 
@@ -817,9 +848,10 @@ def main():
     D = Dist(dist)
 
     def run(cfg_id, st, wu, main_line):
+        dump_dir = args.dump_outputs if main_line else None
         if CONFIGS[cfg_id].get("sliced") is not None:
-            return run_sliced(args, cfg_id, rank, world, local_rank, D, st, wu)
-        return run_sharded(args, cfg_id, rank, world, local_rank, D, st, wu, main_line)
+            return run_sliced(args, cfg_id, rank, world, local_rank, D, st, wu, dump_dir)
+        return run_sharded(args, cfg_id, rank, world, local_rank, D, st, wu, main_line, dump_dir)
 
     line = run(main_cfg, steps, warmup, True)
     secondary = []

@@ -23,12 +23,12 @@ set -euo pipefail
 HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
 REF="${CALS_REFERENCE_DIR:-/root/reference}"
 OUT="$HERE/_ref"
-SP="$(python -c 'import scipy, os; print(os.path.join(os.path.dirname(os.path.dirname(scipy.__file__)), "scipy.libs"))')"
-BLAS="$(ls "$SP"/libscipy_openblas-*.so | head -1)"
 if [ ! -d "$REF/src" ]; then
-  echo "build_ref: $REF not present (GPU box?) -- keeping prebuilt $OUT" >&2
+  echo "build_ref: no reference sources in $REF (set CALS_REFERENCE_DIR) -- keeping whatever $OUT holds" >&2
   exit 0
 fi
+SP="$(python -c 'import scipy, os; print(os.path.join(os.path.dirname(os.path.dirname(scipy.__file__)), "scipy.libs"))')"
+BLAS="$(ls "$SP"/libscipy_openblas-*.so | head -1)"
 mkdir -p "$OUT"
 SRCS=(src/als.cpp src/cals.cpp src/tensor.cpp src/matrix.cpp src/ktensor.cpp src/cals_blas.cpp src/cuda_utils.cpp
       src/utils/utils.cpp src/utils/error.cpp src/utils/mttkrp.cpp src/utils/update.cpp src/multi_ktensor.cpp

@@ -5,6 +5,8 @@ Run in the build container (where /root/reference exists and oracle/build_ref.sh
 Each fixture stores the seeded inputs (tensor + initial models) and the reference's outputs (factors, lambda, error,
 fit_diff, iteration counts, report scalars), so that the oracle and the CUDA path can be checked on machines where the
 reference is not present (the GPU box).  The reference ships no golden vectors of its own (SURVEY.md section 4).
+The exception is `python oracle/make_golden.py full` (main_full): sampled outputs at BASELINE's full sizes, computed by
+the oracle itself, which the fixtures above hold to the reference.
 """
 import os
 import sys
@@ -125,8 +127,62 @@ def main_ls():
     pack("ls_errcheck_3d", X, ms, caseio.run_reference(X, ms, **p), **p)
 
 
+FULL_SAMPLE_ROWS = 4
+
+
+def pack_sampled(name, res, seed):
+    """Full-size outputs, sampled to stay small: per model one column (seeded choice) of every factor at
+    FULL_SAMPLE_ROWS seeded rows per mode, the norm of that whole factor column, its lambda entry, and the model's
+    iteration count, error and fit; plus the report scalars."""
+    rng = np.random.default_rng(seed)
+    N = len(res.models[0].factors)
+    rows = [np.sort(rng.choice(F.shape[0], size=min(FULL_SAMPLE_ROWS, F.shape[0]), replace=False))
+            for F in res.models[0].factors]
+    cols = np.array([int(rng.integers(0, m.rank)) for m in res.models])
+    d = {"iter": res.iters, "n_ktensors": res.n_ktensors, "comp_sum": res.comp_sum, "x_norm": res.x_norm, "cols": cols,
+         "lam": np.array([m.lam[c] for m, c in zip(res.models, cols)]),
+         "iters": np.array([m.iters for m in res.models]), "error": np.array([m.error for m in res.models]),
+         "fit": np.array([m.fit for m in res.models])}
+    for n in range(N):
+        d["rows%d" % n] = rows[n]
+        d["f%d" % n] = np.array([m.factors[n][rows[n], c] for m, c in zip(res.models, cols)])
+        d["colnorm%d" % n] = np.array([np.linalg.norm(m.factors[n][:, c]) for m, c in zip(res.models, cols)])
+    path = os.path.join(OUT, name + ".npz")
+    np.savez_compressed(path, **d)
+    print("wrote", path, os.path.getsize(path) // 1024, "KiB", flush=True)
+
+
+def main_full():
+    """Sampled full-size fixtures for tests/test_full_size.py and the bench contract test, computed by the CPU oracle
+    (oracle/cals_oracle.c, pinned against the reference's own outputs by tests/test_oracle.py) on the seeded inputs
+    those tests build.  `python oracle/make_golden.py full` (about ten minutes on eight cores)."""
+    import oracle
+    sys.path.insert(0, os.path.dirname(OUT))
+    import test_full_size as tfs
+    sys.path.insert(0, os.path.dirname(os.path.dirname(OUT)))
+    import bench
+    for cfg, modes, ranks, seed, Ks in (("config2", (200, 200, 200), [r for r in range(1, 21) for _ in range(10)], 2002,
+                                         (1, 2, 3)),
+                                        ("config4", (80, 80, 80, 80), [r for r in range(1, 31) for _ in range(5)], 4004,
+                                         (1, 2))):
+        X, ms = tfs._driver_inputs(modes, ranks, seed)
+        for K in Ks:
+            res = oracle.cp_cals(X, ms, max_iter=K, force_max_iter=True, buffer_size=sum(ranks))
+            pack_sampled("full_%s_k%d" % (cfg, K), res, seed + K)
+    X, ms = tfs._config3_inputs()
+    res = oracle.cp_cals(X, ms, max_iter=3, force_max_iter=True, buffer_size=sum(m.rank for m in ms))
+    pack_sampled("full_config3_jk_k3", res, 3003)
+    cfg = bench.CONFIGS[2]
+    X, models, jk = bench.workload(cfg, 0)
+    ms = [caseio.Model(factors=fs, jk_mode=j[0], jk_fiber=j[1]) for fs, j in zip(models, jk)]
+    res = oracle.cp_cals(X, ms, max_iter=cfg["als_iters"], force_max_iter=True, buffer_size=sum(cfg["ranks"]))
+    pack_sampled("bench_config2_step", res, 2)
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "ls":
+    if len(sys.argv) > 1 and sys.argv[1] == "full":
+        main_full()
+    elif len(sys.argv) > 1 and sys.argv[1] == "ls":
         main_ls()
     elif len(sys.argv) > 1 and sys.argv[1] == "nnls":
         main_nnls()

@@ -1,5 +1,6 @@
 // Host-only checks of the cals:: containers (no device needed): Tensor / Matrix / Ktensor bookkeeping, normalisation
 // identities, jackknife helpers, linear sum assignment, the model sharding plan.  Prints OK and exits 0 on success.
+// Usage: host_containers_check [DIR]  -- DIR (default /tmp) holds the scratch files of the file-format checks.
 #include <cmath>
 #include <cstdio>
 #include <fstream>
@@ -23,8 +24,9 @@ namespace cals::detail {
 std::vector<std::vector<size_t>> shard_models(const std::vector<dim_t> &ranks, size_t n_parts);
 }
 
-int main() {
+int main(int argc, char **argv) {
   using namespace cals;
+  const std::string scratch = argc > 1 ? argv[1] : "/tmp";
   std::mt19937 gen(0);
   std::uniform_real_distribution<double> dist(-1.0, 1.0);
   auto draw = [&] { return dist(gen); };
@@ -237,24 +239,24 @@ int main() {
 
   // text tensor files (reference src/tensor.cpp:35-65: extents on the first line, values in column-major order)
   {
-    const char *path = "/tmp/cals_b200_tensor_check.txt";
+    const std::string path = scratch + "/cals_b200_tensor_check.txt";
     {
       std::ofstream f(path);
       f << "3 2 2\n";
       for (int i = 0; i < 12; i++)
         f << (i * 0.5 - 1.25) << (i % 4 == 3 ? "\n" : " ");
     }
-    Tensor F{std::string(path)};
+    Tensor F{path};
     REQUIRE(F.get_n_modes() == 3 && F.get_modes()[0] == 3 && F.get_modes()[2] == 2 && F.get_n_elements() == 12);
     REQUIRE(F[0] == -1.25 && F[7] == 2.25 && F[11] == 4.25);
     bool threw = false;
     try {
-      Tensor missing{std::string("/tmp/cals_b200_no_such_file.txt")};
+      Tensor missing{scratch + "/cals_b200_no_such_file.txt"};
     } catch (const std::exception &) {
       threw = true;
     }
     REQUIRE(threw);
-    std::remove(path);
+    std::remove(path.c_str());
   }
 
   // report CSV writers keep the reference's column set (include/cals.h:70-132, include/als.h:70-135)
@@ -275,7 +277,7 @@ int main() {
     rep.mode_times = Matrix(ModeTimers::LENGTH * 3, 2);
     rep.als_times.zero();
     rep.mode_times.zero();
-    const char *path = "/tmp/cals_b200_report_check.csv";
+    const std::string path = scratch + "/cals_b200_report_check.csv";
     rep.print_header(path);
     rep.print_to_file(path);
     std::ifstream f(path);
@@ -291,7 +293,7 @@ int main() {
     REQUIRE(!std::getline(f, extra));
     auto fields = [](const std::string &line) { return std::count(line.begin(), line.end(), ';'); };
     REQUIRE(fields(header) == fields(l1) && fields(header) == 13 + 5 + 6);
-    std::remove(path);
+    std::remove(path.c_str());
 
     AlsReport ar;
     ar.modes = {4, 3, 5};
@@ -312,7 +314,7 @@ int main() {
     REQUIRE(header.rfind("TENSOR_RANK;TENSOR_MODES;KTENSOR_ID;KTENSOR_COMP;UPDATE_METHOD;LINE_SEARCH;MAX_ITERS;ITER;"
                          "NUM_THREADS;TOTAL;FLOPS;ITERATION;", 0) == 0);
     REQUIRE(l1.rfind("0;4-3-5;17;2;unconstrained;0;5;3;", 0) == 0 && fields(header) == fields(l1));
-    std::remove(path);
+    std::remove(path.c_str());
   }
 
   set_threads(6);

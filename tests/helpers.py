@@ -54,6 +54,32 @@ def assert_models_close(got, ref, x_norm, rtol=RTOL, check_iters=True, what=""):
         assert e <= rtol, tag + ": |d error|/||X|| = %.3e" % e
 
 
+def load_sampled(name):
+    """tests/golden/<name>.npz written by oracle/make_golden.py's pack_sampled."""
+    d = np.load(os.path.join(GOLDEN, name + ".npz"))
+    return {k: (d[k].item() if d[k].ndim == 0 else d[k]) for k in d.files}
+
+
+def assert_sampled_models_close(got, want, rtol=RTOL, what=""):
+    """got: objects with .factors .lam .iters .error .fit in queue order; want: load_sampled().  Per model, the stored
+    column's sampled rows of every factor within rtol of that whole column's norm, its lambda entry within rtol, the
+    error within rtol of ||X|| (a cancellation, see assert_models_close), the fit within rtol, equal iteration counts."""
+    cols = want["cols"]
+    assert len(got) == len(cols)
+    xn = want["x_norm"]
+    for i, (g, c) in enumerate(zip(got, cols)):
+        tag = "%s model %d (rank %d)" % (what, i, g.factors[0].shape[1])
+        assert int(g.iters) == int(want["iters"][i]), tag + ": iters %d != %d" % (g.iters, want["iters"][i])
+        for n, F in enumerate(g.factors):
+            e = np.abs(F[want["rows%d" % n], c] - want["f%d" % n][i]).max() / want["colnorm%d" % n][i]
+            assert e <= rtol, tag + ": factor %d column %d sampled rel err %.3e" % (n, c, e)
+        e = abs(g.lam[c] - want["lam"][i]) / abs(want["lam"][i])
+        assert e <= rtol, tag + ": lambda rel err %.3e" % e
+        assert abs(g.error - want["error"][i]) / xn <= rtol, tag + ": |d error|/||X|| = %.3e" % (
+            abs(g.error - want["error"][i]) / xn)
+        assert abs(g.fit - want["fit"][i]) <= rtol, tag + ": fit %.15f != %.15f" % (g.fit, want["fit"][i])
+
+
 def to_ktensors(pkg, models):
     return [pkg.Ktensor([np.array(F, order="F", copy=True) for F in m.factors], None, m.jk_mode, m.jk_fiber)
             for m in models]

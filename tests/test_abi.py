@@ -51,11 +51,11 @@ def test_no_cpu_fallback(pkg):
     assert "no CPU fallback" in str(e.value) or "CUDA" in str(e.value)
 
 
-def test_streamk_bookkeeping_host():
+def test_streamk_bookkeeping_host(tmp_path):
     nvcc = "/usr/local/cuda/bin/nvcc"
     if not os.path.exists(nvcc):
         pytest.skip("nvcc not available")
-    exe = "/tmp/cals_b200_streamk_test"
+    exe = str(tmp_path / "streamk_test")
     subprocess.run([nvcc, "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-o", exe,
                     os.path.join(ROOT, "tests", "cpp", "streamk_host_test.cu")], check=True, capture_output=True)
     out = subprocess.run([exe], capture_output=True, text=True)

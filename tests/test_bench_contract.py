@@ -36,11 +36,12 @@ def test_reference_arm_line():
 
 
 @pytest.mark.gpu
-def test_our_arm_line():
-    """The default invocation (what the driver runs, shortened): headline config 2 with parity against the unmodified
-    reference, CPU baseline, and one `secondary` entry per other BASELINE configuration."""
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3"],
-                         capture_output=True, text=True, timeout=1500)
+def test_our_arm_line(tmp_path):
+    """The default invocation, shortened: headline config 2 with parity against the unmodified reference, CPU
+    baseline, and one `secondary` entry per other BASELINE configuration; --dump-outputs writes the fitted models."""
+    dump = tmp_path / "outputs"
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3",
+                          "--dump-outputs", str(dump)], capture_output=True, text=True, timeout=1500)
     assert out.returncode == 0, out.stderr[-2000:]
     d = _last_json(out.stdout)
     assert BASE_KEYS | {"roofline", "clocks", "gpu_launches"} <= set(d)
@@ -69,6 +70,26 @@ def test_our_arm_line():
         assert s["value"] > 0 and s["unit"] == "model-iterations/s" and s["clocks"]["samples"] > 0
         assert 0.05 < s["roofline"]["frac"] < 1.05 and s["e2e"]["value"] > 0
     assert any("1000x1000x1000" in s["config"]["workload"] for s in sec)
+    import numpy as np
+    got = {p.stem: np.load(p) for p in dump.glob("*.npy")}
+    C = d["config"]["sum_ranks_on_rank0"]
+    shapes = {"factors_mode0": (200, C), "factors_mode1": (200, C), "factors_mode2": (200, C), "lambda": (C,),
+              "iters": (200,), "error": (200,), "fit": (200,)}
+    assert {k: v.shape for k, v in got.items()} == shapes
+    assert all(v.dtype == np.float64 and np.isfinite(v).all() for v in got.values())
+    assert sum(v.nbytes for v in got.values()) <= 64 << 20
+    assert (got["iters"] == d["config"]["als_iters_per_step"]).all() and (got["fit"] < 1).all()
+    # values, model by model in queue order: the dump against the stored outputs of the CPU oracle on the same seeded
+    # workload and iteration count (oracle/make_golden.py full)
+    from types import SimpleNamespace
+    from helpers import RTOL, assert_sampled_models_close, load_sampled
+    ranks = [r for r in range(1, 21) for _ in range(10)]  # bench.CONFIGS[2]
+    assert sum(ranks) == C
+    offs = np.cumsum([0] + ranks)
+    models = [SimpleNamespace(factors=[got["factors_mode%d" % n][:, a:b] for n in range(3)], lam=got["lambda"][a:b],
+                              iters=got["iters"][i], error=got["error"][i], fit=got["fit"][i])
+              for i, (a, b) in enumerate(zip(offs[:-1], offs[1:]))]
+    assert_sampled_models_close(models, load_sampled("bench_config2_step"), rtol=RTOL, what="bench dump")
 
 
 def test_stale_traffic_profile_is_refused(tmp_path, monkeypatch):

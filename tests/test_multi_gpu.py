@@ -160,7 +160,7 @@ def test_multi_gpu_nccl_sharded_cp_cals(tmp_path):
     import torch
     world = min(torch.cuda.device_count(), 4)
     if world < 2:
-        pytest.skip("needs >= 2 GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs")
     _spawn(world, "nccl", True, tmp_path)
     _check_outputs(str(tmp_path), world, 1e-9)
 
@@ -316,7 +316,7 @@ def test_sliced_tensor_over_gpus_matches_oracle(tmp_path):
     import oracle
     world = min(torch.cuda.device_count(), 4)
     if world < 2:
-        pytest.skip("needs >= 2 GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs")
     mp.spawn(_sliced_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
     X, modes, ranks, ms = _sliced_case()
     want = oracle.cp_cals(X, ms, max_iter=5, force_max_iter=True)
