@@ -53,7 +53,7 @@ class Report(C.Structure):
                 ("mttkrp_ms", C.c_double), ("update_ms", C.c_double), ("mttkrp_launches", C.c_uint64),
                 ("kernel_launches", C.c_uint64), ("mttkrp_flops", C.c_double), ("exchange_ms", C.c_double),
                 ("pair_gemm_ms", C.c_double), ("pair_leaf_ms", C.c_double), ("tensor_flops", C.c_double),
-                ("tree", C.c_int32), ("fused_leaf_blocks", C.c_int32)]
+                ("tree", C.c_int32), ("fused_leaf_blocks", C.c_int32), ("sweep_period", C.c_int32)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -218,6 +218,8 @@ class CalsReport:
     ls_performed: int = 0
     ls_failed: int = 0
     pair_node: bool = False  # modes 1 and 2 took their MTTKRP from the shared contraction (csrc/pairnode.cuh)
+    tensor_flops: float = 0.0  # flop of the tensor-sized contractions that actually ran
+    sweep_period: int = 1  # 2: the multi-sweep dimension tree carried a contraction from one iteration to the next
 
 
 class Engine:
@@ -539,7 +541,8 @@ def cp_cals(X: np.ndarray, ktensors: Sequence[Ktensor], params: CalsParams, *, e
                           ktensor_comp_sum=rep.ktensor_comp_sum, tol=params.tol, total_time=rep.total_time,
                           device_ms=rep.device_ms, mttkrp_ms=rep.mttkrp_ms, update_ms=rep.update_ms,
                           mttkrp_launches=rep.mttkrp_launches, kernel_launches=rep.kernel_launches,
-                          ls_performed=lsp, ls_failed=lsf, pair_node=bool(rep.tree))
+                          ls_performed=lsp, ls_failed=lsf, pair_node=bool(rep.tree), tensor_flops=rep.tensor_flops,
+                          sweep_period=rep.sweep_period)
     finally:
         if own:
             eng.close()

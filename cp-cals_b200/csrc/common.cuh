@@ -61,6 +61,12 @@ struct SchedState {
   // their narrow instances on [C_main, C).  C_main == C unless narrow_on and the tail qualifies.
   int C_main;
   int narrow_on; // set by the host per run
+  // Multi-sweep dimension tree (engine.cu: run_loop): an even pass leaves T = X x_1 A_1 behind for the mode-0 update of
+  // the next pass.  carry_ok: this pass is odd and the scheduler moved no column, so that T still matches the buffer;
+  // otherwise mode 0 runs its own MTTKRP.
+  int carry_ok;
+  int carry_pad_;
+  unsigned long long contraction_cols; // sum over executed passes of C x the tensor-sized contractions the pass ran
 };
 
 // eviction predicate + iteration counter (reference src/cals.cpp:336-347); called by exactly one thread per model

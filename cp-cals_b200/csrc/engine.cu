@@ -52,21 +52,24 @@ struct Buffers {
   MttkrpGeom mg[CALS_MAX_MODES];
   int wm[CALS_MAX_MODES];
   PlanArgs plans{}; // per-mode work partition tables (device memory) + the inputs of mttkrp_make_plan
-  // pair nodes (pairnode.cuh): two modes that take their MTTKRP from one shared contraction T.  3 modes: one node
-  // (modes 1, 2; T from pair_gemm_kernel).  4 modes: two nodes (modes 0, 1 and modes 2, 3); their T comes from
-  // mttkrp_dmma_kernel run on a 3-way view of the tensor, set up in the slots n_modes + k of maps / mg / wm / plans.
+  // pair nodes (pairnode.cuh): two modes that take their MTTKRP from one shared contraction T.  3 modes: node k
+  // contracts mode k (T from pair_gemm_kernel, rows (i_{k+1}, i_{k+2})); the one-sweep schedule uses node 0 (modes 1, 2)
+  // only, the multi-sweep schedule (msdt) all three, which share one T and one Gp.  4 modes: two nodes (modes 0, 1 and
+  // modes 2, 3); their T comes from mttkrp_dmma_kernel run on a 3-way view of the tensor, set up in the slots
+  // n_modes + k of maps / mg / wm / plans.
   struct PairNode {
     PairGeom pg{};
     double *T = nullptr; // (E1 * E2) x cols
-    double *Gp = nullptr; // fused first leaf: partial results [ceil(E2 / pair_wm)][cols][ldF[mode_fast]]
+    double *Gp = nullptr; // fused first leaf: partial results [ceil(E2 / wm)][cols][ldF[mode_fast]]
     int slot = -1;       // -1: pair_gemm_kernel
+    PairMaps maps;       // pair_gemm_kernel only
+    int wm = 0;          // its tile height
   };
   bool tree = false;
+  bool msdt = false;
   int n_nodes = 0;
-  PairNode node[2];
-  int node_of[CALS_MAX_MODES] = {}; // node that serves mode n, -1: the mode runs its own full MTTKRP
-  PairMaps pmaps;
-  int pair_wm = 0;
+  PairNode node[3];
+  int node_of[CALS_MAX_MODES] = {}; // one-sweep schedule: node that serves mode n, -1: the mode runs its own MTTKRP
   std::vector<void *> allocs;
 };
 
@@ -90,7 +93,8 @@ struct cals_b200_ctx {
   double *Xp = nullptr; // original order, pitch ldX0
   double *Xt = nullptr; // modes 0 and 1 swapped, pitch ldX1
   double *Xq = nullptr; // 4 modes, whole tensor on this device: mode pairs (0,1) and (2,3) exchanged, pitch ldXq
-  int ldX0 = 0, ldX1 = 0, ldXq = 0;
+  double *Xr = nullptr; // 3 modes, multi-sweep schedule: mode order (2, 0, 1), pitch ldXr (made by the first run using it)
+  int ldX0 = 0, ldX1 = 0, ldXq = 0, ldXr = 0;
   double *jk_norms = nullptr; // dims[0]
   double *d_norm = nullptr;
   double x_norm = 0.0;        // host copy of ||X||; valid only when x_norm_valid
@@ -169,8 +173,9 @@ struct cals_b200_ctx {
 
   // one CALS iteration captured as a CUDA graph (the launch parameters do not change between iterations, nor between
   // runs that reuse the same allocations and options)
-  cudaGraphExec_t iter_graph = nullptr;
-  cudaGraphExec_t batch_graph = nullptr; // the same, several iterations per launch
+  // [parity of the first pass]: the multi-sweep schedule alternates two iteration bodies, every other run uses [0] only
+  cudaGraphExec_t iter_graph[2] = {};
+  cudaGraphExec_t batch_graph[2] = {}; // the same, several iterations per launch
   std::vector<long long> iter_graph_key;
   long long alloc_generation = 0; // bumped whenever prepare_run (re)allocates
 
@@ -535,6 +540,111 @@ bool pair_node_wanted(cals_b200_ctx *c) {
   return c->geo.n_modes == 3 || c->Xq != nullptr;
 }
 
+// CALS_B200_MSDT: -1 unset (the extents decide), 0 / 1 forced.  Read per run -- it is part of the allocation signature.
+int msdt_knob() {
+  const char *e = getenv("CALS_B200_MSDT");
+  return e ? (atoi(e) != 0 ? 1 : 0) : -1;
+}
+
+// Shortest mode for which the multi-sweep schedule pays: the contraction over mode c writes T and its leaves read it
+// back, 16 * (nX / I_c) * C bytes against 2 * nX * C flop, so a short contracted mode makes T's traffic as long as the
+// contraction it saves.
+constexpr int MSDT_MIN_EXTENT = 64;
+
+// The multi-sweep schedule (run_loop) needs a 3-mode tensor whole on this device, factors that no line search rewrites
+// behind the carried T, and no narrow column tail (its tiles carry no fused-leaf partials).
+bool msdt_wanted(cals_b200_ctx *c) {
+  static const bool narrow_instance = getenv("CALS_B200_NARROW") != nullptr;
+  const int knob = msdt_knob();
+  if (knob == 0 || c->geo.n_modes != 3 || c->slice_mode >= 0 || c->ls_enabled || narrow_instance)
+    return false;
+  return knob == 1 || std::min({c->xd[0], c->xd[1], c->xd[2]}) >= MSDT_MIN_EXTENT;
+}
+
+int build_xr(cals_b200_ctx *c) {
+  const int I0 = c->xd[0], I1 = c->xd[1], I2 = c->xd[2];
+  c->ldXr = round_up_int(I2, 2);
+  if (!c->Xr)
+    CU_TRY(c, cudaMalloc((void **)&c->Xr, (size_t)c->ldXr * I0 * I1 * 8));
+  dim3 grid((unsigned)(((long long)I0 * I1 + 31) / 32), (unsigned)((I2 + 31) / 32));
+  rot201_copy_kernel<<<grid, 256, 0, c->stream>>>(c->Xp, c->Xr, I0, I1, I2, c->ldX0, c->ldXr);
+  CU_TRY(c, cudaGetLastError());
+  return 0;
+}
+
+// 3 modes: node k contracts mode k, T[(i_f + E1 * i_s), c] = sum_{i_k} X A_k[i_k, c] with f = k+1, s = k+2 (mod 3), read
+// from a 3-D view (i_k, i_f, i_s) of the tensor with mode k contiguous: Xp for k = 0, Xt (storage order i1, i0, i2) with
+// its two outer strides swapped for k = 1, Xr for k = 2.
+int build_pair_node3(cals_b200_ctx *c, Buffers &b, int k, int cols) {
+  const Geom &geo = c->geo;
+  Buffers::PairNode &nd = b.node[k];
+  const int mf = (k + 1) % 3, ms = (k + 2) % 3;
+  PairGeom &pg = nd.pg;
+  pg = PairGeom{};
+  pg.E1 = c->xd[mf];
+  pg.E2 = c->xd[ms];
+  pg.R = pg.E1 * pg.E2;
+  pg.ldT = pg.R;
+  pg.Ip = c->xd[k];
+  pg.mode_fast = mf;
+  pg.mode_slow = ms;
+  pg.off_fast = c->roff[mf];
+  pg.off_slow = c->roff[ms];
+  for (int m = 0; m < 3; m++)
+    pg.ldF[m] = geo.ldF[m];
+  nd.slot = -1;
+  nd.wm = pick_pair_wm(pg.E1, pg.E2, cols, c->sm_count);
+  // m-tile = 8 values of i_f x wm values of i_s (pairnode.cuh): one box of the 3-D view
+  const cuuint64_t I0 = c->xd[0], I1 = c->xd[1];
+  cuuint64_t dx[3] = {(cuuint64_t)pg.Ip, (cuuint64_t)pg.E1, (cuuint64_t)pg.E2}, sx[2];
+  double *base;
+  if (k == 0) {
+    base = c->Xp;
+    sx[0] = (cuuint64_t)c->ldX0 * 8;
+    sx[1] = (cuuint64_t)c->ldX0 * I1 * 8;
+  } else if (k == 1) {
+    base = c->Xt;
+    sx[0] = (cuuint64_t)c->ldX1 * I0 * 8;
+    sx[1] = (cuuint64_t)c->ldX1 * 8;
+  } else {
+    base = c->Xr;
+    sx[0] = (cuuint64_t)c->ldXr * 8;
+    sx[1] = (cuuint64_t)c->ldXr * I0 * 8;
+  }
+  cuuint32_t bx[3] = {(cuuint32_t)KT, 8, (cuuint32_t)nd.wm};
+  if (encode_map(c, &nd.maps.X, base, 3, dx, sx, bx))
+    return 1;
+  // The first leaf rides in the contraction's epilogue (pairnode.cuh) unless its result is a partial sum that goes
+  // to the exchange buffer (sliced tensor over several GPUs).  Measured (fused against separate
+  // pass): config 2 86.5 k against 84.8 k model-iterations/s, config 1 365 k against 341 k; the 8-way shard of
+  // config 2 -- 263 columns, where the TMA-fed slow leaf already streams T at HBM speed and the epilogue is a larger
+  // share of the short tiles -- 57.6 k against 58.0 k, so a narrow buffer over a large T keeps the separate pass.
+  // CALS_B200_FUSED_LEAF=0 / 1 forces either.
+  const int fl = fused_leaf_knob();
+  static const bool narrow_instance = getenv("CALS_B200_NARROW") != nullptr; // (its tiles carry no partials)
+  const bool narrow_big = cols <= LEAF_TMA_MAX_COLS && (size_t)pg.R * cols * 8 > ((size_t)32 << 20);
+  const bool want_fused = fl >= 0 ? fl != 0 : !narrow_big;
+  pg.fuse_slow = (want_fused && !narrow_instance && !(c->slice_mode >= 0 && c->comm_world > 1)) ? 1 : 0;
+  pg.ld_fast = geo.ldF[mf];
+  pg.gp_stride = (long long)cols * geo.ldF[mf];
+  for (int cu = 0; cu < 2; cu++) {
+    if (pg.fuse_slow) { // the slow factor's rows of a tile: [wm rounded up to even] x TILE_N
+      cuuint64_t da[2] = {(cuuint64_t)pg.E2, (cuuint64_t)cols};
+      cuuint64_t sa[1] = {(cuuint64_t)geo.ldF[ms] * 8};
+      cuuint32_t ba[2] = {(cuuint32_t)((nd.wm + 1) & ~1), (cuuint32_t)TILE_N};
+      if (encode_map(c, &nd.maps.A[cu], b.fac.buf[cu][ms] + pg.off_slow, 2, da, sa, ba))
+        return 1;
+    }
+    cuuint64_t d2[2] = {(cuuint64_t)pg.Ip, (cuuint64_t)cols};
+    cuuint64_t s2[1] = {(cuuint64_t)geo.ldF[k] * 8};
+    cuuint32_t b2[2] = {(cuuint32_t)KT, (cuuint32_t)TILE_N}, b2n[2] = {(cuuint32_t)KT, (cuuint32_t)NARROW_COLS};
+    if (encode_map(c, &nd.maps.B[cu], b.fac.buf[cu][k] + c->roff[k], 2, d2, s2, b2) ||
+        encode_map(c, &nd.maps.Bn[cu], b.fac.buf[cu][k] + c->roff[k], 2, d2, s2, b2n))
+      return 1;
+  }
+  return 0;
+}
+
 int alloc_buffers(cals_b200_ctx *c, Buffers &b, int cols, bool with_home_cols, int home_cols) {
   const Geom &geo = c->geo;
   b.cols = cols;
@@ -560,23 +670,54 @@ int alloc_buffers(cals_b200_ctx *c, Buffers &b, int cols, bool with_home_cols, i
   // pair nodes (run buffers only; the single-MTTKRP test hook stays per mode)
   const int N = geo.n_modes;
   b.tree = false;
+  b.msdt = false;
   b.n_nodes = 0;
   for (int n = 0; n < CALS_MAX_MODES; n++)
     b.node_of[n] = -1;
   if (with_home_cols && pair_node_wanted(c)) {
-    // 3 modes: node 0 = modes (1,2).  4 modes: node 0 = modes (0,1), node 1 = modes (2,3).
-    const int n_nodes = N == 3 ? 1 : 2;
-    size_t need = 0;
-    for (int k = 0; k < n_nodes; k++) {
-      const int mf = N == 3 ? 1 : 2 * k;
-      need += (size_t)c->xd[mf] * c->xd[mf + 1] * (size_t)cols * 8;
-    }
     size_t free_b = 0, total_b = 0;
     CU_TRY(c, cudaMemGetInfo(&free_b, &total_b));
-    if (2 * need + ((size_t)2 << 30) < free_b) { // T plus, for 4 modes, a partial-tile workspace of similar size
-      for (int k = 0; k < n_nodes; k++) {
+    auto fits = [&](size_t need) { // T plus, for 4 modes, a partial-tile workspace of similar size
+      return 2 * need + ((size_t)2 << 30) < free_b;
+    };
+    if (N == 3) {
+      // one-sweep schedule: node 0 = modes (1,2).  Multi-sweep: nodes 0, 1, 2 with one T and one Gp of the largest size,
+      // and the (2, 0, 1) copy of the tensor.
+      const size_t R0 = (size_t)c->xd[1] * c->xd[2];
+      const size_t R_max = std::max({R0, (size_t)c->xd[2] * c->xd[0], (size_t)c->xd[0] * c->xd[1]});
+      const size_t xr_bytes = c->Xr ? 0 : (size_t)round_up_int(c->xd[2], 2) * c->xd[0] * c->xd[1] * 8;
+      b.msdt = msdt_wanted(c) && fits(R_max * cols * 8 + xr_bytes);
+      if (b.msdt || fits(R0 * cols * 8)) {
+        if (b.msdt && !c->Xr && build_xr(c))
+          return 1;
+        b.n_nodes = b.msdt ? 3 : 1;
+        double *T = nullptr;
+        // + 2: the leaf kernels' bulk copies read 16-byte granules and may touch one double past the last row
+        if (dev_alloc(c, &T, (b.msdt ? R_max : R0) * cols + 2, b.allocs))
+          return 1;
+        size_t gp = 0;
+        for (int k = 0; k < b.n_nodes; k++) {
+          if (build_pair_node3(c, b, k, cols))
+            return 1;
+          const PairGeom &pg = b.node[k].pg;
+          b.node[k].T = T;
+          if (pg.fuse_slow)
+            gp = std::max(gp, (size_t)(pg.E2 + b.node[k].wm - 1) / b.node[k].wm * (size_t)pg.gp_stride);
+        }
+        double *Gp = nullptr;
+        if (gp > 0 && dev_alloc(c, &Gp, gp, b.allocs))
+          return 1;
+        for (int k = 0; k < b.n_nodes; k++)
+          b.node[k].Gp = Gp;
+        b.node_of[1] = b.node_of[2] = 0;
+        b.tree = true;
+      }
+    } else if (fits(((size_t)c->xd[0] * c->xd[1] + (size_t)c->xd[2] * c->xd[3]) * cols * 8)) {
+      // 4 modes: node 0 = modes (0,1), node 1 = modes (2,3)
+      b.n_nodes = 2;
+      for (int k = 0; k < b.n_nodes; k++) {
         Buffers::PairNode &nd = b.node[k];
-        const int mf = N == 3 ? 1 : 2 * k;
+        const int mf = 2 * k;
         nd.pg = PairGeom{};
         nd.pg.E1 = c->xd[mf];
         nd.pg.E2 = c->xd[mf + 1];
@@ -588,66 +729,22 @@ int alloc_buffers(cals_b200_ctx *c, Buffers &b, int cols, bool with_home_cols, i
         nd.pg.off_slow = c->roff[mf + 1];
         for (int m = 0; m < N; m++)
           nd.pg.ldF[m] = geo.ldF[m];
-        nd.slot = N == 3 ? -1 : N + k;
+        nd.slot = N + k;
         // + 2: the leaf kernels' bulk copies read 16-byte granules and may touch one double past the last row
         if (dev_alloc(c, &nd.T, (size_t)nd.pg.R * cols + 2, b.allocs))
           return 1;
         b.node_of[mf] = b.node_of[mf + 1] = k;
       }
-      b.n_nodes = n_nodes;
       b.tree = true;
-      for (int k = 0; k < n_nodes; k++) { // dynamic shared memory of the TMA-fed leaf kernel (ring of stages)
-        const size_t ss = leaf_slow_smem(b.node[k].pg.E2);
-        if (ss > c->leaf_slow_attr) {
-          CU_TRY(c, cudaFuncSetAttribute(pair_leaf_slow_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss));
-          c->leaf_slow_attr = ss;
-        }
-      }
-      if (N == 3) {
-        PairGeom &pg = b.node[0].pg;
-        pg.Ip = c->xd[0];
-        b.pair_wm = pick_pair_wm(pg.E1, pg.E2, cols, c->sm_count);
-        // m-tile = 8 values of i1 x pair_wm values of i2 (pairnode.cuh): one box of the 3-D view
-        cuuint64_t dx[3] = {(cuuint64_t)c->xd[0], (cuuint64_t)pg.E1, (cuuint64_t)pg.E2};
-        cuuint64_t sx[2] = {(cuuint64_t)c->ldX0 * 8, (cuuint64_t)c->ldX0 * pg.E1 * 8};
-        cuuint32_t bx[3] = {(cuuint32_t)KT, 8, (cuuint32_t)b.pair_wm};
-        if (encode_map(c, &b.pmaps.X, c->Xp, 3, dx, sx, bx))
-          return 1;
-        // The first leaf rides in the contraction's epilogue (pairnode.cuh) unless its result is a partial sum that goes
-        // to the exchange buffer (sliced tensor over several GPUs).  Measured (gpurun_out/exp31, fused against separate
-        // pass): config 2 86.5 k against 84.8 k model-iterations/s, config 1 365 k against 341 k; the 8-way shard of
-        // config 2 -- 263 columns, where the TMA-fed slow leaf already streams T at HBM speed and the epilogue is a larger
-        // share of the short tiles -- 57.6 k against 58.0 k, so a narrow buffer over a large T keeps the separate pass.
-        // CALS_B200_FUSED_LEAF=0 / 1 forces either.
-        const int fl = fused_leaf_knob();
-        static const bool narrow_instance = getenv("CALS_B200_NARROW") != nullptr; // (its tiles carry no partials)
-        const bool narrow_big = cols <= LEAF_TMA_MAX_COLS && (size_t)pg.R * cols * 8 > ((size_t)32 << 20);
-        const bool want_fused = fl >= 0 ? fl != 0 : !narrow_big;
-        pg.fuse_slow = (want_fused && !narrow_instance && !(c->slice_mode >= 0 && c->comm_world > 1)) ? 1 : 0;
-        pg.ld_fast = geo.ldF[pg.mode_fast];
-        pg.gp_stride = (long long)cols * geo.ldF[pg.mode_fast];
-        if (pg.fuse_slow) {
-          const size_t E2b = (size_t)(pg.E2 + b.pair_wm - 1) / b.pair_wm;
-          if (dev_alloc(c, &b.node[0].Gp, E2b * (size_t)pg.gp_stride, b.allocs))
-            return 1;
-          for (int cu = 0; cu < 2; cu++) { // the slow factor's rows of a tile: [pair_wm rounded up to even] x TILE_N
-            cuuint64_t da[2] = {(cuuint64_t)pg.E2, (cuuint64_t)cols};
-            cuuint64_t sa[1] = {(cuuint64_t)geo.ldF[pg.mode_slow] * 8};
-            cuuint32_t ba[2] = {(cuuint32_t)((b.pair_wm + 1) & ~1), (cuuint32_t)TILE_N};
-            if (encode_map(c, &b.pmaps.A[cu], b.fac.buf[cu][pg.mode_slow] + pg.off_slow, 2, da, sa, ba))
-              return 1;
-          }
-        }
-        for (int cu = 0; cu < 2; cu++) {
-          cuuint64_t d2[2] = {(cuuint64_t)c->xd[0], (cuuint64_t)cols};
-          cuuint64_t s2[1] = {(cuuint64_t)geo.ldF[0] * 8};
-          cuuint32_t b2[2] = {(cuuint32_t)KT, (cuuint32_t)TILE_N}, b2n[2] = {(cuuint32_t)KT, (cuuint32_t)NARROW_COLS};
-          if (encode_map(c, &b.pmaps.B[cu], b.fac.buf[cu][0], 2, d2, s2, b2) ||
-              encode_map(c, &b.pmaps.Bn[cu], b.fac.buf[cu][0], 2, d2, s2, b2n))
-            return 1;
-        }
-      } else if (build_node_slots(c, b))
+      if (build_node_slots(c, b))
         return 1;
+    }
+    for (int k = 0; k < b.n_nodes; k++) { // dynamic shared memory of the TMA-fed leaf kernel (ring of stages)
+      const size_t ss = leaf_slow_smem(b.node[k].pg.E2);
+      if (ss > c->leaf_slow_attr) {
+        CU_TRY(c, cudaFuncSetAttribute(pair_leaf_slow_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss));
+        c->leaf_slow_attr = ss;
+      }
     }
   }
 
@@ -699,7 +796,7 @@ int alloc_buffers(cals_b200_ctx *c, Buffers &b, int cols, bool with_home_cols, i
   return 0;
 }
 
-template <int WM> int launch_pair_gemm_wm(cals_b200_ctx *c, Buffers &b, bool attr_only) {
+template <int WM> int launch_pair_gemm_wm(cals_b200_ctx *c, Buffers &b, const Buffers::PairNode &nd, bool attr_only) {
   auto kern = pair_gemm_kernel<WM, WN_FIXED>;
   constexpr int smem = PairCfg<WM, WN_FIXED>::SMEM_BYTES;
   if (!c->pair_attr_done[WM]) {
@@ -712,47 +809,51 @@ template <int WM> int launch_pair_gemm_wm(cals_b200_ctx *c, Buffers &b, bool att
     c->pair_attr_done[8 + WM] = true;
   }
   if (!attr_only) {
-    CU_TRY(c, launch_chain(c, kern, dim3(c->sm_count), dim3(MTTKRP_THREADS), (size_t)smem, b.pmaps, b.node[0].pg,
-                           (const SchedState *)c->d_st, b.node[0].T, b.node[0].Gp));
+    CU_TRY(c, launch_chain(c, kern, dim3(c->sm_count), dim3(MTTKRP_THREADS), (size_t)smem, nd.maps, nd.pg,
+                           (const SchedState *)c->d_st, nd.T, nd.Gp));
     if (b.narrow)
-      CU_TRY(c, launch_chain(c, kern_n, dim3(c->sm_count), dim3(MTTKRP_THREADS), (size_t)smem, b.pmaps, b.node[0].pg,
-                             (const SchedState *)c->d_st, b.node[0].T, b.node[0].Gp));
+      CU_TRY(c, launch_chain(c, kern_n, dim3(c->sm_count), dim3(MTTKRP_THREADS), (size_t)smem, nd.maps, nd.pg,
+                             (const SchedState *)c->d_st, nd.T, nd.Gp));
   }
   return 0;
 }
 
-// T = X_(0)^T A_0 (attr_only: just make sure the kernel's shared-memory attribute is set, outside of a graph capture)
-int launch_pair_gemm(cals_b200_ctx *c, Buffers &b, bool attr_only = false) {
-  switch (b.pair_wm) {
+// T of 3-mode node k: the tensor contracted over mode k (attr_only: just make sure the kernel's shared-memory attribute
+// is set, outside of a graph capture)
+int launch_pair_gemm(cals_b200_ctx *c, Buffers &b, int k, bool attr_only = false) {
+  const Buffers::PairNode &nd = b.node[k];
+  switch (nd.wm) {
   case 4:
-    return launch_pair_gemm_wm<4>(c, b, attr_only);
+    return launch_pair_gemm_wm<4>(c, b, nd, attr_only);
   case 5:
-    return launch_pair_gemm_wm<5>(c, b, attr_only);
+    return launch_pair_gemm_wm<5>(c, b, nd, attr_only);
   case 6:
-    return launch_pair_gemm_wm<6>(c, b, attr_only);
+    return launch_pair_gemm_wm<6>(c, b, nd, attr_only);
   case 7:
-    return launch_pair_gemm_wm<7>(c, b, attr_only);
+    return launch_pair_gemm_wm<7>(c, b, nd, attr_only);
   default:
-    return launch_pair_gemm_wm<8>(c, b, attr_only);
+    return launch_pair_gemm_wm<8>(c, b, nd, attr_only);
   }
 }
 
 double *exchange_data(cals_b200_ctx *c);
 
-// MTTKRP of mode n from the T of its pair node
-int launch_pair_leaf(cals_b200_ctx *c, Buffers &b, int n, bool exchange) {
-  const Buffers::PairNode &nd = b.node[b.node_of[n]];
-  const PairGeom &pg = nd.pg;
+// MTTKRP of mode n (one of the two modes of node k) from the node's T.  carried: the second leaf of a T made in the
+// previous pass, which runs only when the scheduler found that T still valid (SchedState::carry_ok).
+int launch_pair_leaf(cals_b200_ctx *c, Buffers &b, int k, int n, bool exchange, bool carried = false) {
+  const Buffers::PairNode &nd = b.node[k];
+  PairGeom pg = nd.pg;
+  pg.carried = carried ? 1 : 0;
   LeafExchange x{};
   x.xbuf = exchange ? exchange_data(c) : nullptr;
   x.xcap = (unsigned long long)c->xcap;
   x.seq_base = c->seq_base;
   x.n_modes = c->geo.n_modes;
   if (n == pg.mode_fast && pg.fuse_slow && nd.slot < 0 && !exchange) {
-    // the contraction's epilogue has left ceil(E2 / pair_wm) partial results per element
+    // the contraction's epilogue has left ceil(E2 / wm) partial results per element
     dim3 grid((unsigned)((pg.E1 + 255) / 256), (unsigned)b.cols);
     CU_TRY(c, launch_chain(c, pair_partial_reduce_kernel, grid, dim3(256), (size_t)0, pg, (const SchedState *)c->d_st,
-                           (const double *)nd.Gp, (pg.E2 + b.pair_wm - 1) / b.pair_wm, b.G));
+                           (const double *)nd.Gp, (pg.E2 + nd.wm - 1) / nd.wm, b.G));
   } else if (n == pg.mode_fast) {
     dim3 grid((unsigned)b.cols, (unsigned)((pg.E1 + 255) / 256));
     if (b.cols <= LEAF_TMA_MAX_COLS) // narrow grid: one TMA-fed stream per column
@@ -812,7 +913,10 @@ int join_prefactor(cals_b200_ctx *c, int n) {
 }
 
 template <int WM>
-int launch_dmma(cals_b200_ctx *c, Buffers &b, int n, int C_override, bool exchange, bool skip_reduce, double *out) {
+int launch_dmma(cals_b200_ctx *c, Buffers &b, int n, int C_override, bool exchange, bool skip_reduce, double *out,
+                bool carry_fallback) {
+  MttkrpGeom mg = b.mg[n];
+  mg.carry_fallback = carry_fallback ? 1 : 0;
   auto kern = mttkrp_dmma_kernel<WM, WN_FIXED, false>;
   auto kern_n = mttkrp_dmma_kernel<WM, WN_FIXED, true>;
   if (set_dmma_attr<WM>(c))
@@ -822,10 +926,10 @@ int launch_dmma(cals_b200_ctx *c, Buffers &b, int n, int C_override, bool exchan
   const int tail = (C_override > 0 && b.narrow) ? narrow_cols(C_override) : 0;
   const int C_main_ov = C_override > 0 ? C_override - tail : 0;
   if (C_override <= 0 || C_main_ov > 0)
-    CU_TRY(c, launch_chain(c, kern, dim3(G), dim3(MTTKRP_THREADS), (size_t)smem_bytes<WM>(), b.maps[n], b.mg[n],
+    CU_TRY(c, launch_chain(c, kern, dim3(G), dim3(MTTKRP_THREADS), (size_t)smem_bytes<WM>(), b.maps[n], mg,
                            (const SchedState *)c->d_st, b.fac, (const int *)b.plans.plan[n], b.ws, C_main_ov, 0));
   if (b.narrow && (C_override <= 0 || tail > 0))
-    CU_TRY(c, launch_chain(c, kern_n, dim3(G), dim3(MTTKRP_THREADS), (size_t)smem_bytes<WM>(), b.maps[n], b.mg[n],
+    CU_TRY(c, launch_chain(c, kern_n, dim3(G), dim3(MTTKRP_THREADS), (size_t)smem_bytes<WM>(), b.maps[n], mg,
                            (const SchedState *)c->d_st, b.fac, (const int *)b.plans.plan_narrow[n], b.ws_n, C_override,
                            C_main_ov));
   if (skip_reduce) // the update kernel sums the partial tiles itself
@@ -838,7 +942,7 @@ int launch_dmma(cals_b200_ctx *c, Buffers &b, int n, int C_override, bool exchan
   }
   const int cols = C_override > 0 ? C_override : b.cols;
   dim3 rg((cols + 31) / 32, (b.mg[n].In + REDUCE_ROWS - 1) / REDUCE_ROWS);
-  CU_TRY(c, launch_chain(c, mttkrp_reduce_kernel<8 * WM, TILE_N>, rg, dim3(256), (size_t)0, b.mg[n],
+  CU_TRY(c, launch_chain(c, mttkrp_reduce_kernel<8 * WM, TILE_N>, rg, dim3(256), (size_t)0, mg,
                          (const SchedState *)c->d_st, (const int *)b.plans.plan[n], (const double *)b.ws, out, G,
                          C_override, exchange ? exchange_data(c) : (double *)nullptr, (unsigned long long)c->xcap,
                          (unsigned long long)c->seq_base, c->geo.n_modes, (const int *)b.plans.plan_narrow[n],
@@ -847,8 +951,9 @@ int launch_dmma(cals_b200_ctx *c, Buffers &b, int n, int C_override, bool exchan
 }
 
 // n < n_modes: MTTKRP of mode n into G.  n >= n_modes: contraction of a pair node's slot into `out` (its T).
+// carry_fallback: the kernels run only when the carried T is not valid (SchedState::carry_ok == 0).
 int launch_mttkrp(cals_b200_ctx *c, Buffers &b, int n, int C_override, int variant, bool exchange = false,
-                  bool skip_reduce = false, double *out = nullptr) {
+                  bool skip_reduce = false, double *out = nullptr, bool carry_fallback = false) {
   if (!out)
     out = b.G;
   if (variant == CALS_B200_MTTKRP_NAIVE) {
@@ -874,15 +979,15 @@ int launch_mttkrp(cals_b200_ctx *c, Buffers &b, int n, int C_override, int varia
   }
   switch (b.wm[n]) {
   case 4:
-    return launch_dmma<4>(c, b, n, C_override, exchange, skip_reduce, out);
+    return launch_dmma<4>(c, b, n, C_override, exchange, skip_reduce, out, carry_fallback);
   case 5:
-    return launch_dmma<5>(c, b, n, C_override, exchange, skip_reduce, out);
+    return launch_dmma<5>(c, b, n, C_override, exchange, skip_reduce, out, carry_fallback);
   case 6:
-    return launch_dmma<6>(c, b, n, C_override, exchange, skip_reduce, out);
+    return launch_dmma<6>(c, b, n, C_override, exchange, skip_reduce, out, carry_fallback);
   case 7:
-    return launch_dmma<7>(c, b, n, C_override, exchange, skip_reduce, out);
+    return launch_dmma<7>(c, b, n, C_override, exchange, skip_reduce, out, carry_fallback);
   default:
-    return launch_dmma<8>(c, b, n, C_override, exchange, skip_reduce, out);
+    return launch_dmma<8>(c, b, n, C_override, exchange, skip_reduce, out, carry_fallback);
   }
 }
 
@@ -897,12 +1002,14 @@ int ensure_dummy_state(cals_b200_ctx *c) {
 }
 
 void drop_iteration_graph(cals_b200_ctx *c) {
-  if (c->iter_graph)
-    cudaGraphExecDestroy(c->iter_graph);
-  if (c->batch_graph)
-    cudaGraphExecDestroy(c->batch_graph);
-  c->iter_graph = nullptr;
-  c->batch_graph = nullptr;
+  for (int p = 0; p < 2; p++) {
+    if (c->iter_graph[p])
+      cudaGraphExecDestroy(c->iter_graph[p]);
+    if (c->batch_graph[p])
+      cudaGraphExecDestroy(c->batch_graph[p]);
+    c->iter_graph[p] = nullptr;
+    c->batch_graph[p] = nullptr;
+  }
   c->iter_graph_key.clear();
 }
 
@@ -956,7 +1063,9 @@ void release_tensor(cals_b200_ctx *c) {
     cudaFree(c->jk_norms);
   if (c->Xq)
     cudaFree(c->Xq);
-  c->Xp = c->Xt = c->Xq = c->jk_norms = nullptr;
+  if (c->Xr)
+    cudaFree(c->Xr);
+  c->Xp = c->Xt = c->Xq = c->Xr = c->jk_norms = nullptr;
   c->have_tensor = false;
 }
 
@@ -1046,6 +1155,8 @@ int install_tensor(cals_b200_ctx *c, int n_modes, const uint64_t *modes, const d
     dim3 grid((I0 + 31) / 32, (I2 + 31) / 32, (unsigned)std::min<long long>((long long)I1 * I3, 65535));
     halves_swap_kernel<<<grid, 256, 0, c->stream>>>(c->Xp, c->Xq, I0, I1, I2, I3, c->ldX0, c->ldXq);
   }
+  if (c->Xr && build_xr(c)) // same shape as before: the (2, 0, 1) copy that an earlier run made follows the new values
+    return 1;
   // norms: one pass over Xp
   if (!c->jk_norms)
     CU_TRY(c, cudaMalloc((void **)&c->jk_norms, (size_t)(I0 + 1) * 8));
@@ -1105,6 +1216,7 @@ int prepare_run(cals_b200_ctx *c) {
   sig.push_back(c->ls_enabled ? 1 + c->ls_method : 0);
   sig.push_back(c->pair_node);
   sig.push_back(fused_leaf_knob());
+  sig.push_back(msdt_knob());
   for (int m = 0; m < M; m++)
     sig.push_back(c->hmodels[m].rank);
   const bool reuse = !c->run_sig.empty() && sig == c->run_sig && c->d_models && c->bufs.cols == c->buffer_cols;
@@ -1270,6 +1382,28 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
   // pair nodes: two modes share one contraction of the tensor (pairnode.cuh)
   const bool tree = b.tree && c->variant == CALS_B200_MTTKRP_DMMA;
   auto node_of = [&](int n) { return tree ? b.node_of[n] : -1; };
+  // Multi-sweep dimension tree (3 modes, pairnode.cuh): node k contracts mode k and serves modes k+1 and k+2.
+  //   even pass:  node 2 (T = X x_2 A_2): mode 0 (first leaf), mode 1 (second leaf);
+  //               node 1 (T = X x_1 A_1): mode 2 (first leaf); its second leaf is mode 0 of the NEXT pass
+  //   odd pass:   mode 0 from that carried T, or -- when the scheduler moved columns (SchedState::carry_ok == 0) -- from
+  //               its own MTTKRP: both sit in the odd iteration body and the one whose turn it is not returns at once;
+  //               node 0 (T = X x_0 A_0): mode 1 (first leaf), mode 2 (second leaf)
+  // Every mode sees the factors the per-mode MTTKRP sees; three contractions per two passes instead of four.  Pass 0 of
+  // every run is even, so nothing is carried into a run.
+  const bool msdt = tree && b.msdt && !c->ls_enabled && !fused_reduce;
+  // per mode and parity: node whose T serves the mode (-1: its own MTTKRP), whether that T is made right before
+  struct Source {
+    int node;
+    bool contract, carried;
+  };
+  auto source = [&](int n, int odd) -> Source {
+    if (msdt && !odd)
+      return {n == 2 ? 1 : 2, n != 1, false};
+    if (msdt)
+      return {n == 0 ? 1 : 0, n == 1, n == 0};
+    const int k = node_of(n);
+    return {k, k >= 0 && n == b.node[k].pg.mode_fast, false};
+  };
 
   // tuning aid: CALS_B200_UPDATE_PROF=1 prints the phase times of the update kernel's slowest CTA per mode after the run
   static const bool update_prof = getenv("CALS_B200_UPDATE_PROF") != nullptr;
@@ -1418,8 +1552,10 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
     size_t e0, e1;
     int kind;
     long long iteration;
+    int odd; // parity of the iteration body that recorded it
   };
   std::vector<Window> timed;
+  int body_odd = 0; // parity of the iteration body being enqueued
 
   uint64_t launches = 1, mttkrp_launches = 0;
   auto t0 = std::chrono::steady_clock::now();
@@ -1439,19 +1575,27 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
   };
   auto window = [&](size_t e0, size_t e1, int kind) {
     if (c->timing)
-      timed.push_back({e0, e1, kind, it});
+      timed.push_back({e0, e1, kind, it, body_odd});
   };
-  // everything one CALS iteration launches, in stream order
-  int launches_per_iteration = 0;
+  // everything one CALS iteration launches, in stream order; odd: the odd body of the multi-sweep schedule
+  int launches_per_iteration[2] = {0, 0};
   bool pref_on = false; // decided below, before the first call of enqueue_iteration
-  auto enqueue_iteration = [&](bool count) -> int {
+  auto enqueue_iteration = [&](bool count, int odd) -> int {
     int n_launch = 0;
+    body_odd = odd;
     auto chain_ok = [&](cudaError_t e, const char *what) {
       if (e != cudaSuccess)
         fail(c, "launch of %s failed: %s", what, cudaGetErrorString(e));
       return e == cudaSuccess;
     };
-    sched_kernel<<<1, 32, 0, s>>>(sp); // first kernel of the iteration: plain stream order after the previous iteration
+    SchedParams spi = sp;
+    spi.carry = msdt && odd;
+    spi.contractions = 0; // (the fallback MTTKRP of an odd pass is counted by the scheduler itself)
+    for (int n = 0; n < N; n++) {
+      const Source src = source(n, odd);
+      spi.contractions += (src.node < 0 || src.contract) ? 1 : 0;
+    }
+    sched_kernel<<<1, 32, 0, s>>>(spi); // first kernel of the iteration: plain stream order after the previous iteration
     if (!chain_ok(launch_chain(c, move_kernel, move_grid, dim3(256), (size_t)0, geo, b.fac, (const SchedState *)c->d_st,
                                (const int *)c->d_gather, (const int *)c->d_evict),
                   "move_kernel"))
@@ -1464,12 +1608,13 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
     for (int n = 0; n < N; n++) {
       const size_t e0 = mark();
       size_t e1;
-      if (node_of(n) >= 0) {
-        const Buffers::PairNode &nd = b.node[node_of(n)];
+      const Source src = source(n, odd);
+      if (src.node >= 0) {
+        const Buffers::PairNode &nd = b.node[src.node];
         size_t el = e0;
-        if (n == nd.pg.mode_fast) { // first mode of the pair: refresh T
+        if (src.contract) { // first mode served by this T: make it
           if (nd.slot < 0) {
-            if (launch_pair_gemm(c, b))
+            if (launch_pair_gemm(c, b, src.node))
               return -1;
             n_launch += b.narrow ? 2 : 1;
           } else {
@@ -1485,7 +1630,7 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
             return -1;
           n_launch++;
         }
-        if (launch_pair_leaf(c, b, n, exchange))
+        if (launch_pair_leaf(c, b, src.node, n, exchange, src.carried))
           return -1;
         n_launch++;
         if (exchange) {
@@ -1496,6 +1641,14 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
         }
         e1 = mark();
         window(el, e1, T_PAIR_LEAF); // includes the exchange
+        if (src.carried) { // ... or, when the columns moved, mode 0's own MTTKRP (no exchange: the tensor is whole here)
+          if (launch_mttkrp(c, b, n, 0, c->variant, false, false, nullptr, true))
+            return -1;
+          n_launch += 2;
+          const size_t e2 = mark();
+          window(e1, e2, T_MTTKRP);
+          e1 = e2;
+        }
       } else {
         if (pref_on) { // ... or next to the partial-tile reduction (launch_dmma forks between its two kernels)
           if (c->variant == CALS_B200_MTTKRP_NAIVE) {
@@ -1539,7 +1692,7 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
       }
     }
     if (count)
-      launches_per_iteration = n_launch;
+      launches_per_iteration[odd] = n_launch;
     return n_launch;
   };
 
@@ -1564,10 +1717,8 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
     for (int n = 0; n < N; n++)
       if (c->variant == CALS_B200_MTTKRP_DMMA && ensure_dmma_attr(c, b.wm[n]))
         return 1;
-    if (tree && b.node[0].slot < 0 && launch_pair_gemm(c, b, true))
-      return 1;
     for (int k = 0; tree && k < b.n_nodes; k++)
-      if (b.node[k].slot >= 0 && ensure_dmma_attr(c, b.wm[b.node[k].slot]))
+      if (b.node[k].slot < 0 ? launch_pair_gemm(c, b, k, true) : ensure_dmma_attr(c, b.wm[b.node[k].slot]))
         return 1;
     return 0;
   };
@@ -1577,8 +1728,9 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
   // every launch adds microseconds of idle time, which inflates the windows of short kernels (a 140 us contraction of an
   // 8-way shard was reported as 175 us).
   const bool timed_graph = c->timing && !exchange && !graphs_off && !c->ls_enabled;
-  cudaGraphExec_t tgraph = nullptr;
+  cudaGraphExec_t tgraph[2] = {};
   double tsum[5] = {0, 0, 0, 0, 0};
+  const int n_bodies = msdt ? 2 : 1; // iteration bodies: even (and odd)
   // The head of every update (H, Cholesky, block inverses) on a forked branch of the iteration graph, off the critical
   // path (update.cuh: prefactor_kernel).  OFF unless CALS_B200_PREFACTOR=1: measured on the B200 the fork / join edges
   // and the kernel running next to the leaf cost more than the 17 k cycles they take out of the update kernel (8-way
@@ -1610,58 +1762,73 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
       up[n].pref_stride = c->pref_stride;
     }
   }
+  auto free_tgraphs = [&]() {
+    for (auto &g : tgraph)
+      if (g)
+        cudaGraphExecDestroy(g);
+  };
   if (timed_graph) {
     if (prepare_capture())
       return 1;
-    get_event(c, ev_next + 16 * (size_t)(N + 2)); // create the events of one iteration before the capture begins
-    cudaGraph_t graph = nullptr;
-    CU_TRY(c, cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    capturing_timed = true;
-    const int rc = enqueue_iteration(true);
-    capturing_timed = false;
-    cudaError_t ce = cudaStreamEndCapture(s, &graph);
-    if (rc < 0 || ce != cudaSuccess) {
-      if (graph)
-        cudaGraphDestroy(graph);
-      return rc < 0 ? 1 : fail(c, "cudaStreamEndCapture (timed) failed: %s", cudaGetErrorString(ce));
+    // create the events of the iteration bodies before the capture begins
+    get_event(c, ev_next + 16 * (size_t)(N + 2) * n_bodies);
+    for (int odd = 0; odd < n_bodies; odd++) {
+      cudaGraph_t graph = nullptr;
+      CU_TRY(c, cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+      capturing_timed = true;
+      const int rc = enqueue_iteration(true, odd);
+      capturing_timed = false;
+      cudaError_t ce = cudaStreamEndCapture(s, &graph);
+      if (rc < 0 || ce != cudaSuccess) {
+        if (graph)
+          cudaGraphDestroy(graph);
+        free_tgraphs();
+        return rc < 0 ? 1 : fail(c, "cudaStreamEndCapture (timed) failed: %s", cudaGetErrorString(ce));
+      }
+      ce = cudaGraphInstantiate(&tgraph[odd], graph, 0);
+      cudaGraphDestroy(graph);
+      if (ce != cudaSuccess) {
+        free_tgraphs();
+        return fail(c, "cudaGraphInstantiate (timed) failed: %s", cudaGetErrorString(ce));
+      }
     }
-    ce = cudaGraphInstantiate(&tgraph, graph, 0);
-    cudaGraphDestroy(graph);
-    if (ce != cudaSuccess)
-      return fail(c, "cudaGraphInstantiate (timed) failed: %s", cudaGetErrorString(ce));
   }
   if (use_graph) {
     std::vector<long long> key = {c->alloc_generation, (long long)c->flags, c->ls_enabled, c->ls_method, c->variant,
-                                  (long long)max_live, fused_reduce ? 1 : 0, tree ? 1 : 0, c->pdl ? 1 : 0, graph_batch, pref_on ? 1 : 0};
-    const bool same_graph = c->iter_graph && c->iter_graph_key.size() == key.size() + 1 &&
+                                  (long long)max_live, fused_reduce ? 1 : 0, tree ? 1 : 0, c->pdl ? 1 : 0, graph_batch,
+                                  pref_on ? 1 : 0, msdt ? 1 : 0};
+    const bool same_graph = c->iter_graph[0] && c->iter_graph_key.size() == key.size() + 2 &&
                             std::equal(key.begin(), key.end(), c->iter_graph_key.begin());
     if (!same_graph) {
       drop_iteration_graph(c);
       if (prepare_capture())
         return 1;
-      // two graphs: one CALS iteration, and GRAPH_BATCH iterations back to back (used while the number of passes still
-      // to run is known to be at least that, see below)
-      for (int which = 0; which < 2; which++) {
-        cudaGraph_t graph = nullptr;
-        CU_TRY(c, cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-        int rc = 0;
-        for (int k = 0; k < (which == 0 ? 1 : graph_batch) && rc >= 0; k++)
-          rc = enqueue_iteration(true);
-        cudaError_t ce = cudaStreamEndCapture(s, &graph);
-        if (rc < 0 || ce != cudaSuccess) {
-          if (graph)
-            cudaGraphDestroy(graph);
-          return rc < 0 ? 1 : fail(c, "cudaStreamEndCapture failed: %s", cudaGetErrorString(ce));
+      // per body parity, two graphs: one CALS iteration, and GRAPH_BATCH iterations back to back starting with that
+      // parity (used while the number of passes still to run is known to be at least that, see below)
+      for (int odd = 0; odd < n_bodies; odd++)
+        for (int which = 0; which < 2; which++) {
+          cudaGraph_t graph = nullptr;
+          CU_TRY(c, cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+          int rc = 0;
+          for (int k = 0; k < (which == 0 ? 1 : graph_batch) && rc >= 0; k++)
+            rc = enqueue_iteration(true, msdt ? (odd + k) & 1 : 0);
+          cudaError_t ce = cudaStreamEndCapture(s, &graph);
+          if (rc < 0 || ce != cudaSuccess) {
+            if (graph)
+              cudaGraphDestroy(graph);
+            return rc < 0 ? 1 : fail(c, "cudaStreamEndCapture failed: %s", cudaGetErrorString(ce));
+          }
+          ce = cudaGraphInstantiate(which == 0 ? &c->iter_graph[odd] : &c->batch_graph[odd], graph, 0);
+          cudaGraphDestroy(graph);
+          if (ce != cudaSuccess)
+            return fail(c, "cudaGraphInstantiate failed: %s", cudaGetErrorString(ce));
         }
-        ce = cudaGraphInstantiate(which == 0 ? &c->iter_graph : &c->batch_graph, graph, 0);
-        cudaGraphDestroy(graph);
-        if (ce != cudaSuccess)
-          return fail(c, "cudaGraphInstantiate failed: %s", cudaGetErrorString(ce));
-      }
       c->iter_graph_key = key;
-      c->iter_graph_key.push_back(launches_per_iteration);
+      c->iter_graph_key.push_back(launches_per_iteration[0]);
+      c->iter_graph_key.push_back(launches_per_iteration[1]);
     } else {
-      launches_per_iteration = (int)c->iter_graph_key.back();
+      launches_per_iteration[0] = (int)c->iter_graph_key[key.size()];
+      launches_per_iteration[1] = (int)c->iter_graph_key[key.size() + 1];
     }
   }
 
@@ -1673,14 +1840,17 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
       c->total_cols <= c->buffer_cols && !c->ls_enabled)
     known_passes = (long long)c->max_iter + 1;
   for (;; it++) {
+    const int odd = msdt ? (int)(it & 1) : 0; // the host picks the body by the parity of the pass
     if (timed_graph) {
-      CU_TRY(c, cudaGraphLaunch(tgraph, s));
-      launches += launches_per_iteration;
+      CU_TRY(c, cudaGraphLaunch(tgraph[odd], s));
+      launches += launches_per_iteration[odd];
       mttkrp_launches += N;
       CU_TRY(c, cudaStreamSynchronize(s));
       const bool drained = *(volatile int *)&c->h_flags[0] != 0; // this pass found the queue empty: no work in it
       if (!drained)
         for (auto &t : timed) {
+          if (t.odd != odd)
+            continue;
           float e = 0;
           cudaEventElapsedTime(&e, get_event(c, t.e0), get_event(c, t.e1));
           tsum[t.kind] += e;
@@ -1690,15 +1860,16 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
       continue;
     }
     if (use_graph && known_passes > 0 && it + graph_batch <= known_passes && graph_batch > 1) {
-      CU_TRY(c, cudaGraphLaunch(c->batch_graph, s));
-      launches += (uint64_t)launches_per_iteration * graph_batch;
+      CU_TRY(c, cudaGraphLaunch(c->batch_graph[odd], s));
+      for (int k = 0; k < graph_batch; k++)
+        launches += (uint64_t)launches_per_iteration[msdt ? (odd + k) & 1 : 0];
       mttkrp_launches += (uint64_t)N * (graph_batch - 1);
       it += graph_batch - 1;
     } else if (use_graph) {
-      CU_TRY(c, cudaGraphLaunch(c->iter_graph, s));
-      launches += launches_per_iteration;
+      CU_TRY(c, cudaGraphLaunch(c->iter_graph[odd], s));
+      launches += launches_per_iteration[odd];
     } else {
-      const int rc = enqueue_iteration(false);
+      const int rc = enqueue_iteration(false, odd);
       if (rc < 0)
         return 1;
       launches += rc;
@@ -1720,8 +1891,7 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
   CU_TRY(c, cudaStreamSynchronize(s));
   CU_TRY(c, cudaGetLastError());
   auto t1 = std::chrono::steady_clock::now();
-  if (tgraph)
-    cudaGraphExecDestroy(tgraph);
+  free_tgraphs();
 
   if (update_prof && c->d_update_prof) {
     std::vector<long long> h((size_t)N * max_live * 16);
@@ -1772,16 +1942,14 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
     rep->mttkrp_launches = real_mttkrp;
     rep->kernel_launches = launches;
     rep->mttkrp_flops = 2.0 * (double)c->nX * (double)N * (double)st.col_iter_sum;
-    // flop that actually ran on the tensor cores: with the pair node two contractions per iteration instead of N
+    // flop that actually ran on the tensor cores: the scheduler counts the contractions of every executed pass (pair
+    // nodes: two per iteration instead of N; multi-sweep schedule: three per two iterations, plus the fallback MTTKRPs)
     rep->tree = tree ? 1 : 0;
     rep->fused_leaf_blocks = (tree && N == 3 && b.node[0].pg.fuse_slow && !exchange)
-                                 ? (b.node[0].pg.E2 + b.pair_wm - 1) / b.pair_wm
+                                 ? (b.node[0].pg.E2 + b.node[0].wm - 1) / b.node[0].wm
                                  : 0;
-    int contractions = 0;
-    for (int n = 0; n < N; n++)
-      contractions += node_of(n) < 0 ? 1 : 0;
-    contractions += tree ? b.n_nodes : 0;
-    rep->tensor_flops = 2.0 * (double)c->nX * (double)contractions * (double)st.col_iter_sum;
+    rep->tensor_flops = 2.0 * (double)c->nX * (double)st.contraction_cols;
+    rep->sweep_period = msdt ? 2 : 1;
     if (c->timing) {
       // passes launched after the queue drained (host run-ahead) are not counted
       double sum[5] = {0, 0, 0, 0, 0};

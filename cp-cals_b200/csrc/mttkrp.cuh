@@ -62,6 +62,7 @@ struct MttkrpGeom {
   // rows [off, off + extent) of the sliced mode's factor.  Offsets are 0 everywhere else.
   int outer_off[CALS_MAX_OUTER]; // row offset into the factor of every outer mode
   int g_row_off;                 // row offset of this device's G rows (non-zero only when mode == sliced mode)
+  int carry_fallback; // runs only when SchedState::carry_ok is 0 (mode 0 in an odd pass of the multi-sweep schedule)
 };
 
 struct MttkrpMaps {
@@ -489,7 +490,7 @@ mttkrp_dmma_kernel(const __grid_constant__ MttkrpMaps maps, const MttkrpGeom g, 
   const int C = C_override > 0 ? C_override : (NARROW ? st->C : st->C_main);
   const int c_lo = NARROW ? (C_override > 0 ? C_lo_override : st->C_main) : 0; // first column of the narrow tail
   const int cur = C_override > 0 ? 0 : st->cur;
-  if (C - c_lo <= 0)
+  if (C - c_lo <= 0 || (g.carry_fallback && st->carry_ok))
     return;
   const PlanView pv = plan_view(plan, gridDim.x);
   const int lo = pv.cta_lo[blockIdx.x], hi = pv.cta_lo[blockIdx.x + 1];
@@ -768,7 +769,7 @@ mttkrp_reduce_kernel(const MttkrpGeom g, const SchedState *__restrict__ st, cons
     G = xbuf + (seq & 1ull) * xcap;
   }
   const int c0 = blockIdx.x * 32, m0 = blockIdx.y * REDUCE_ROWS;
-  if (c0 >= C)
+  if (c0 >= C || (g.carry_fallback && st->carry_ok))
     return;
   __shared__ double t[REDUCE_ROWS][33];
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5; // 256 threads: ty in 0..7

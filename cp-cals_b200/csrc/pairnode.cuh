@@ -17,6 +17,12 @@
 // association differs.  An ALS iteration then costs two tensor-sized contractions instead of three (four).  This is the
 // reference's own two-step idea (mttkrp_twostep0/1, src/utils/mttkrp.cpp:460-553: "mode1/TS0 uses the same T as mode0/TS0")
 // carried across modes; T lives in HBM.  CalsParams::mttkrp_method == MTTKRP selects one full MTTKRP per mode instead.
+//
+// Multi-sweep dimension tree (3 modes, engine.cu: run_loop; Ma & Solomonik, IPDPS 2021): the same kernels contract any
+// mode c -- T = X x_c A_c, rows (i_{c+1}, i_{c+2}), first leaf to mode c+1, second leaf to mode c+2 (indices mod 3) --
+// from a 3-D view of the tensor with mode c contiguous (PairGeom / PairMaps carry the roles).  Even passes contract
+// modes 2 and 1, odd passes mode 0; the second leaf of the mode-1 contraction updates mode 0 in the NEXT pass, so two
+// passes cost three contractions instead of four.
 #pragma once
 #include "mttkrp.cuh"
 
@@ -61,6 +67,7 @@ struct PairGeom {
   int fuse_slow;
   int ld_fast;         // ldF[mode_fast] (a plain field: the kernels index no parameter array at run time)
   long long gp_stride; // doubles between the partial results of consecutive b2 (= buffer columns * ldF[mode_fast])
+  int carried; // second leaf from a T of the previous pass: runs only when SchedState::carry_ok (engine.cu: run_loop)
 };
 
 // T = X_(0)^T A_0.  Persistent CTAs over the (m-tile, n-tile) grid, m-tile fastest, so that the CTAs running at the
@@ -340,7 +347,7 @@ pair_leaf_fast_kernel(const PairGeom g, const SchedState *__restrict__ st, const
   pdl_enter();
   const int C = st->C, cur = st->cur;
   const int c = blockIdx.x;
-  if (c >= C)
+  if (c >= C || (g.carried && !st->carry_ok))
     return;
   G = leaf_output(G, x, st, g.mode_slow);
   extern __shared__ double wcol[]; // E1

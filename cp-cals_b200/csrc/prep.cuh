@@ -2,6 +2,7 @@
 //
 //   pad_copy_kernel        X (dense, mode 0 fastest)  ->  Xp with the fastest dimension padded to an even pitch
 //   swap01_copy_kernel     X -> Xt with modes 0 and 1 swapped (mode 1 fastest), pitch padded to even
+//   rot201_copy_kernel     3-mode X -> Xr with mode order (2, 0, 1) (mode 2 fastest), pitch padded to even
 //   halves_swap_kernel     4-mode X -> Xq with the mode pairs (0,1) and (2,3) exchanged (mode 2 fastest), pitch padded
 //   rowsumsq_*             per mode-0 index sums of squares in ONE pass over X, from which both
 //                            ||X||          Tensor::norm                       reference include/tensor.h:196
@@ -67,6 +68,34 @@ __global__ void swap01_copy_kernel(const double *__restrict__ X, double *__restr
       if (i0 < I0 && i1 < ld1)
         Xd[(long long)i0 * ld1 + i1] = (i1 < I1) ? t[tx][aa] : 0.0;
     }
+  }
+}
+
+// 3 modes: Xr[i2 + ldr * (i0 + I0 * i1)] = Xp[i0 + ld0 * (i1 + I1 * i2)], mode order (2, 0, 1): the contraction over mode
+// 2 of the multi-sweep dimension tree reads it with mode 2 contiguous (engine.cu).  The transpose of X viewed as the
+// (I0*I1) x I2 matrix; grid = (ceil(I0*I1 / 32), ceil(I2 / 32))
+__global__ void rot201_copy_kernel(const double *__restrict__ Xp, double *__restrict__ Xr, int I0, int I1, int I2,
+                                   int ld0, int ldr) {
+  __shared__ double t[32][33];
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5; // 256 threads
+  const long long R = (long long)I0 * I1, r0 = (long long)blockIdx.x * 32;
+  const int k0 = blockIdx.y * 32;
+  for (int kk = ty; kk < 32; kk += 8) {
+    const long long r = r0 + tx;
+    const int i2 = k0 + kk;
+    double v = 0.0;
+    if (r < R && i2 < I2) {
+      const long long i1 = r / I0, i0 = r - i1 * I0;
+      v = Xp[i0 + (long long)ld0 * (i1 + (long long)I1 * i2)];
+    }
+    t[kk][tx] = v;
+  }
+  __syncthreads();
+  for (int rr = ty; rr < 32; rr += 8) {
+    const long long r = r0 + rr;
+    const int i2 = k0 + tx;
+    if (r < R && i2 < ldr)
+      Xr[i2 + (long long)ldr * r] = i2 < I2 ? t[tx][rr] : 0.0;
   }
 }
 

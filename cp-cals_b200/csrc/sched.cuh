@@ -26,6 +26,9 @@ struct SchedParams {
   int *host_flags; // mapped pinned host memory: [0] done, [1] global_iter (low 31 bits), [2] n_live
   PlanArgs plans;  // MTTKRP work partition per mode, rebuilt whenever the live column count changes
   unsigned *iter_cols; // [ITER_LOG_CAP] active column count of every executed iteration (CalsReport::cols)
+  int contractions;    // tensor-sized contractions of this pass (not counting the fallback MTTKRP below)
+  int carry;           // odd pass of the multi-sweep schedule: mode 0 takes the carried T, or its own MTTKRP when the
+                       // columns change in this pass (SchedState::carry_ok)
 };
 constexpr int ITER_LOG_CAP = 65536;
 
@@ -45,6 +48,7 @@ __global__ void __launch_bounds__(32) sched_kernel(const SchedParams p) {
     sh_C_before = st->C;
     if (st->done) {
       st->changed = 0;
+      st->carry_ok = 0;
     } else {
       const int B = st->buffer_cols;
       bool changed = false;
@@ -148,6 +152,8 @@ __global__ void __launch_bounds__(32) sched_kernel(const SchedParams p) {
       st->changed = changed ? 1 : 0;
       if (changed)
         st->cur ^= 1;
+      const bool carry_ok = p.carry && !changed; // a moved column or a flipped buffer no longer matches the carried T
+      st->carry_ok = carry_ok ? 1 : 0;
       if (n_live == 0 && next >= n_models) {
         st->done = 1;
       } else {
@@ -155,6 +161,7 @@ __global__ void __launch_bounds__(32) sched_kernel(const SchedParams p) {
           p.iter_cols[st->global_iter] = (unsigned)col;
         st->global_iter += 1; // reference: rep.iter counts executed loop bodies (src/cals.cpp:175-176)
         st->col_iter_sum += (unsigned long long)col;
+        st->contraction_cols += (unsigned long long)col * (unsigned)(p.contractions + (p.carry && !carry_ok ? 1 : 0));
       }
       p.host_flags[1] = (int)(st->global_iter & 0x7fffffff);
       p.host_flags[2] = n_live;

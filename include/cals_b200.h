@@ -59,6 +59,9 @@ typedef struct cals_b200_report {
   int32_t tree;              /* 1 when the pair node was used by this run */
   int32_t fused_leaf_blocks; /* > 0: the first leaf of the 3-mode pair node rode in the contraction's epilogue; the number
                                 of partial results per element that pair_partial_reduce_kernel summed (ceil(I2 / tile)) */
+  int32_t sweep_period;      /* 2: the multi-sweep dimension tree ran (3 modes: the contraction over mode 1 also serves
+                                mode 0 of the next iteration, three tensor-sized contractions per two iterations);
+                                1: every iteration runs the same contractions */
 } cals_b200_report;
 
 typedef struct cals_b200_model_stats {
