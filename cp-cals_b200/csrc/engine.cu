@@ -23,6 +23,7 @@
 #include "prep.cuh"
 #include "sched.cuh"
 #include "update.cuh"
+#include "wide.cuh"
 
 using namespace calsb200;
 
@@ -117,6 +118,8 @@ struct cals_b200_ctx {
   std::vector<HostModel> hmodels;
   std::vector<ModelDesc> hdesc;
   int total_cols = 0, max_rank = 0;
+  // models above the shared-memory update kernel's rank bound (wide.cuh); narrow_rank: largest rank at or below it
+  int narrow_rank = 0, n_wide = 0, wide_min_rank = 0, wide_max_rank = 0;
   long long gram_doubles = 0;
   bool uploaded = false;
   bool results_fresh = false;
@@ -188,6 +191,11 @@ struct cals_b200_ctx {
   cudaStream_t stream2 = nullptr;
   cudaEvent_t ev_fork[CALS_MAX_MODES] = {}, ev_join[CALS_MAX_MODES] = {};
   double *d_pref = nullptr; // run allocation: max_live slots of pref_stride doubles
+  // wide-model workspace (wide.cuh): wide_slots slots of wide_slot_stride doubles
+  double *d_wide = nullptr;
+  long long wide_slot_stride = 0;
+  int wide_slots = 0, wide_ldw = 0, wide_y_rows = 0;
+  bool wide_attr_done = false;
   long long pref_stride = 0;
   size_t prefactor_attr_smem = 0;
   PrefactorParams pf[CALS_MAX_MODES];
@@ -1024,6 +1032,7 @@ void release_run(cals_b200_ctx *c) {
   c->d_live = c->d_live_tmp = c->d_gather = c->d_evict = nullptr;
   c->d_gram = c->d_lambda = nullptr;
   c->d_pref = nullptr;
+  c->d_wide = nullptr;
   c->d_active = nullptr;
   for (int n = 0; n < CALS_MAX_MODES; n++)
     c->ls_prev[n] = c->ls_backup[n] = nullptr;
@@ -1194,6 +1203,65 @@ int ensure_host_norm(cals_b200_ctx *c) {
   return 0;
 }
 
+// Shared-memory layout of model_update_kernel for rank R, extent `rows` and the given update method; false when rank R
+// does not fit.  The one place that knows the kernel's budget: run_loop sizes the launch with it and
+// narrow_rank_bound() derives the largest rank the kernel accepts from it.
+struct UpdateSmemPlan {
+  int nnls_warps, chunk_rows, table_off;
+  size_t smem;
+};
+bool plan_update_smem(int R, int rows, bool nnls, UpdateSmemPlan *pl) {
+  const int R8 = round_up_int(R, 8); // the small matrices and the staged chunk are zero-padded to a multiple of 8
+  size_t fixed = ((size_t)2 * R8 * R8 + 4 * R + 64 + 2 * STAT_SEGS * R) * 8; // H / L, block inverses / Gramian,
+  // column statistics, 1 / diag(L), diag(H), reduction scratch, statistics candidates
+  const size_t budget = 200 * 1024;
+  pl->nnls_warps = 0;
+  if (nnls) { // per working warp: 5R + R*R doubles and 2R + 1 ints of scratch
+    const size_t per_warp = ((size_t)5 * R + (size_t)R * R + (size_t)(2 * R + 2) / 2 + 1) * 8;
+    int nw = UPDATE_THREADS / 32;
+    while (nw > 1 && fixed + nw * per_warp + (size_t)36 * R8 * 8 > budget)
+      nw >>= 1;
+    pl->nnls_warps = nw;
+    fixed += nw * per_warp;
+  }
+  if (fixed + (size_t)36 * R8 * 8 > budget)
+    return false;
+  int cr = round_up_int(rows, 32);
+  // behind the staged chunk: tile lookup tables of the fused reduction, (R + chunk rows) ints
+  auto tables = [&](int rows_) { return (size_t)((R + rows_ + 1) / 2 + 1) * 8; };
+  while (cr >= 32 && fixed + (size_t)(cr + 4) * R8 * 8 + tables(cr) > budget)
+    cr -= 32;
+  if (cr < 32)
+    return false;
+  pl->chunk_rows = cr;
+  pl->table_off = (int)((fixed + (size_t)(cr + 4) * R8 * 8) / 8);
+  pl->smem = fixed + (size_t)(cr + 4) * R8 * 8 + tables(cr);
+  return true;
+}
+
+// Largest rank the shared-memory update kernel accepts (96 unconstrained, 80 NNLS); models above it are "wide" and
+// take the multi-CTA path of wide.cuh (unconstrained only).  The fit does not depend on the extent: a long mode only
+// shortens the staged chunk, down to 32 rows.
+int narrow_rank_bound(bool nnls) {
+  auto largest = [](bool nn) {
+    UpdateSmemPlan pl;
+    int r = 0;
+    while (plan_update_smem(r + 1, 1, nn, &pl))
+      r++;
+    return r;
+  };
+  static const int bound[2] = {largest(false), largest(true)}; // thread-safe one-time initialisation
+  return bound[nnls ? 1 : 0];
+}
+
+// NNLS keeps the rank bound: its row-wise active-set solver needs R^2 scratch per warp in shared memory.
+int check_nnls_rank(cals_b200_ctx *c, int model, int rank) {
+  const int bound = narrow_rank_bound(true);
+  if ((c->flags & CALS_B200_NNLS) && rank > bound)
+    return fail(c, "model %d has rank %d, above %d, the largest rank the NNLS update supports", model, rank, bound);
+  return 0;
+}
+
 // Upload the queued models and allocate every run-time structure.
 int prepare_run(cals_b200_ctx *c) {
   if (!c->have_tensor)
@@ -1226,7 +1294,8 @@ int prepare_run(cals_b200_ctx *c) {
   }
 
   c->hdesc.assign(M, ModelDesc{});
-  int col = 0, max_rank = 0;
+  const int bound = narrow_rank_bound(false);
+  int col = 0, max_rank = 0, narrow_rank = 0, n_wide = 0, wide_min = 0, wide_max = 0;
   long long goff = 0, aoff = 0, sum_rows = 0;
   for (int n = 0; n < N; n++)
     sum_rows += geo.dims[n];
@@ -1248,9 +1317,21 @@ int prepare_run(cals_b200_ctx *c) {
     goff += (long long)N * hm.rank * hm.rank;
     aoff += sum_rows * hm.rank;
     max_rank = std::max(max_rank, hm.rank);
+    if (check_nnls_rank(c, m, hm.rank))
+      return 1;
+    if (hm.rank > bound) {
+      wide_min = n_wide ? std::min(wide_min, hm.rank) : hm.rank;
+      wide_max = std::max(wide_max, hm.rank);
+      n_wide++;
+    } else
+      narrow_rank = std::max(narrow_rank, hm.rank);
   }
   c->total_cols = col;
   c->max_rank = max_rank;
+  c->narrow_rank = narrow_rank;
+  c->n_wide = n_wide;
+  c->wide_min_rank = wide_min;
+  c->wide_max_rank = wide_max;
   c->gram_doubles = goff;
   c->active_bytes = aoff;
   if ((long long)c->h_active.size() != aoff)
@@ -1271,9 +1352,22 @@ int prepare_run(cals_b200_ctx *c) {
       if (dev_alloc(c, &c->home0[n], (size_t)geo.ldF[n] * c->total_cols, c->run_allocs))
         return 1;
     {
-      const long long ld8 = round_up_int(max_rank, 8);
+      const long long ld8 = round_up_int(std::max(narrow_rank, 1), 8); // wide models never take the prefactor branch
       c->pref_stride = 2 * ld8 * ld8 + 2 * ld8 + 2;
       if (dev_alloc(c, &c->d_pref, (size_t)std::min(M, c->buffer_cols) * (size_t)c->pref_stride, c->run_allocs))
+        return 1;
+    }
+    c->wide_slots = 0;
+    if (n_wide > 0) { // one workspace slot per wide model that can be live at the same time
+      int max_dim = 0;
+      for (int n = 0; n < N; n++)
+        max_dim = std::max(max_dim, geo.dims[n]);
+      c->wide_ldw = round_up_int(wide_max, WIDE_NB);
+      c->wide_y_rows = round_up_int(max_dim, WIDE_NB);
+      const long long ldw = c->wide_ldw;
+      c->wide_slot_stride = 3 * ldw * ldw + (long long)c->wide_y_rows * ldw + 2 * ldw;
+      c->wide_slots = std::min(n_wide, c->buffer_cols / wide_min);
+      if (dev_alloc(c, &c->d_wide, (size_t)c->wide_slots * (size_t)c->wide_slot_stride, c->run_allocs))
         return 1;
     }
     if (c->ls_enabled) {
@@ -1376,8 +1470,9 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
   // everywhere (config 1: 307.5 k vs 302 k model-iterations/s) -- a few update CTAs cannot pull tens of partial tiles
   // per element as fast as the whole chip -- so the fused form only runs when CALS_B200_FUSED_REDUCE=1 asks for it.
   static const bool fusion_forced = getenv("CALS_B200_FUSED_REDUCE") != nullptr;
+  // A wide model's update reads G, so a queue that holds one always runs the separate reduce, which materialises G.
   const bool fused_reduce = c->variant == CALS_B200_MTTKRP_DMMA && !(c->slice_mode >= 0 && c->comm_world > 1) &&
-                            !fusion_off && fusion_forced && !b.narrow;
+                            !fusion_off && fusion_forced && !b.narrow && c->n_wide == 0;
 
   // pair nodes: two modes share one contraction of the tensor (pairnode.cuh)
   const bool tree = b.tree && c->variant == CALS_B200_MTTKRP_DMMA;
@@ -1424,33 +1519,17 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
     u.n_modes = N;
     u.rows = geo.dims[n];
     u.ld = geo.ldF[n];
-    const int R = c->max_rank;
-    const int R8 = round_up_int(R, 8); // the small matrices and the staged chunk are zero-padded to a multiple of 8
-    size_t fixed = ((size_t)2 * R8 * R8 + 4 * R + 64 + 2 * STAT_SEGS * R) * 8; // H / L, block inverses / Gramian,
-    // column statistics, 1 / diag(L), diag(H), reduction scratch, statistics candidates
-    const size_t budget = 200 * 1024;
+    // sized for the largest narrow rank; the CTAs of wide models return at once
+    const int R = std::max(c->narrow_rank, 1);
     u.nnls = (c->flags & CALS_B200_NNLS) ? 1 : 0;
-    u.nnls_warps = 0;
-    if (u.nnls) { // per working warp: 5R + R*R doubles and 2R + 1 ints of scratch
-      const size_t per_warp = ((size_t)5 * R + (size_t)R * R + (size_t)(2 * R + 2) / 2 + 1) * 8;
-      int nw = UPDATE_THREADS / 32;
-      while (nw > 1 && fixed + nw * per_warp + (size_t)36 * R8 * 8 > budget)
-        nw >>= 1;
-      u.nnls_warps = nw;
-      fixed += nw * per_warp;
-    }
-    if (fixed + (size_t)36 * R8 * 8 > budget)
+    UpdateSmemPlan pl;
+    if (!plan_update_smem(R, u.rows, u.nnls, &pl))
       return fail(c, "rank %d too large for the shared-memory update kernel", R);
-    int cr = round_up_int(u.rows, 32);
-    // behind the staged chunk: tile lookup tables of the fused reduction, (R + chunk rows) ints
-    auto tables = [&](int rows_) { return (size_t)((R + rows_ + 1) / 2 + 1) * 8; };
-    while (fixed + (size_t)(cr + 4) * R8 * 8 + tables(cr) > budget)
-      cr -= 32;
-    if (cr < 32)
-      return fail(c, "rank %d too large for the shared-memory update kernel", R);
+    const int cr = pl.chunk_rows;
+    u.nnls_warps = pl.nnls_warps;
     u.chunk_rows = cr;
     u.chunk_pitch = cr + 4; // = 4 mod 16 doubles: the DMMA fragment loads of the update kernel are bank-conflict free
-    u.table_off = (int)((fixed + (size_t)(cr + 4) * R8 * 8) / 8);
+    u.table_off = pl.table_off;
     u.max_rank = R;
     u.G = b.G;
     u.F[0] = b.fac.buf[0][n];
@@ -1474,8 +1553,47 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
     u.pref = nullptr;
     u.pref_stride = 0;
     u.prof = c->d_update_prof ? c->d_update_prof + (size_t)n * max_live * 16 : nullptr;
-    up_smem[n] = fixed + (size_t)(cr + 4) * R8 * 8 + tables(cr);
+    up_smem[n] = pl.smem;
   }
+  // models of rank above the bound: the multi-CTA update of wide.cuh after the narrow one, per mode
+  const bool has_wide = c->n_wide > 0;
+  const bool has_narrow = c->n_wide < M;
+  WideParams wp[CALS_MAX_MODES];
+  for (int n = 0; n < N && has_wide; n++) {
+    WideParams &w = wp[n];
+    w.mode = n;
+    w.n_modes = N;
+    w.rows = geo.dims[n];
+    w.ld = geo.ldF[n];
+    w.bound = narrow_rank_bound(false);
+    w.G = b.G;
+    w.F[0] = b.fac.buf[0][n];
+    w.F[1] = b.fac.buf[1][n];
+    w.gram_pool = c->d_gram;
+    w.lambda_home = c->d_lambda;
+    w.x_norms_jk = c->jk_norms;
+    w.models = c->d_models;
+    w.live = c->d_live;
+    w.st = c->d_st;
+    w.ws = c->d_wide;
+    w.slot_stride = c->wide_slot_stride;
+    w.ldw = c->wide_ldw;
+    w.y_rows = c->wide_y_rows;
+  }
+  if (has_wide && !c->wide_attr_done) {
+    CU_TRY(c, cudaFuncSetAttribute(wide_factor_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)WIDE_FACTOR_SMEM));
+    CU_TRY(c, cudaFuncSetAttribute(wide_solve_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)WIDE_TILE_SMEM));
+    CU_TRY(c, cudaFuncSetAttribute(wide_solve_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)WIDE_TILE_SMEM));
+    CU_TRY(c, cudaFuncSetAttribute(wide_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WIDE_TILE_SMEM));
+    c->wide_attr_done = true;
+  }
+  if ((c->flags & CALS_B200_NNLS) && c->max_rank > narrow_rank_bound(true)) // options changed after prepare_run
+    for (int m = 0; m < M; m++)
+      if (check_nnls_rank(c, m, c->hmodels[m].rank))
+        return 1;
   {
     size_t mx = 0;
     for (int n = 0; n < N; n++)
@@ -1673,13 +1791,30 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
       }
       if (pref_on && join_prefactor(c, n))
         return -1;
-      if (!chain_ok(up[n].nnls ? launch_chain(c, model_update_kernel<true>, dim3(max_live), dim3(UPDATE_THREADS),
-                                              up_smem[n], up[n])
-                               : launch_chain(c, model_update_kernel<false>, dim3(max_live), dim3(UPDATE_THREADS),
-                                              up_smem[n], up[n]),
-                    "model_update_kernel"))
-        return -1;
-      n_launch++;
+      if (has_narrow) {
+        if (!chain_ok(up[n].nnls ? launch_chain(c, model_update_kernel<true>, dim3(max_live), dim3(UPDATE_THREADS),
+                                                up_smem[n], up[n])
+                                 : launch_chain(c, model_update_kernel<false>, dim3(max_live), dim3(UPDATE_THREADS),
+                                                up_smem[n], up[n]),
+                      "model_update_kernel"))
+          return -1;
+        n_launch++;
+      }
+      if (has_wide) {
+        const int S = c->wide_slots, CT = c->wide_ldw / WIDE_NB, RT = (geo.dims[n] + WIDE_NB - 1) / WIDE_NB;
+        wide_factor_kernel<<<dim3(WIDE_CLUSTER, S), WIDE_THREADS, WIDE_FACTOR_SMEM, s>>>(wp[n]);
+        wide_solve_kernel<0><<<dim3(RT * CT, S), WIDE_THREADS, WIDE_TILE_SMEM, s>>>(wp[n]);
+        wide_solve_kernel<1><<<dim3(RT * CT, S), WIDE_THREADS, WIDE_TILE_SMEM, s>>>(wp[n]);
+        wide_stats_kernel<<<dim3(c->wide_ldw / WIDE_STAT_COLS, S), WIDE_THREADS, 0, s>>>(wp[n]);
+        wide_gram_kernel<<<dim3(CT * (CT + 1) / 2, S), WIDE_THREADS, WIDE_TILE_SMEM, s>>>(wp[n]);
+        n_launch += 5;
+        if (n == N - 1) {
+          wide_error_kernel<<<S, WIDE_THREADS, 0, s>>>(wp[n]);
+          n_launch++;
+        }
+        if (!chain_ok(cudaGetLastError(), "the wide-model update kernels"))
+          return -1;
+      }
       window(e1, mark(), T_UPDATE);
     }
     if (c->ls_enabled) {
@@ -1739,7 +1874,7 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
   pref_on = (use_graph || timed_graph) && pref_wanted && !(c->flags & CALS_B200_NNLS) && !c->ls_enabled && !fused_reduce &&
             c->d_pref != nullptr;
   {
-    const long long ld8 = round_up_int(c->max_rank, 8);
+    const long long ld8 = round_up_int(std::max(c->narrow_rank, 1), 8);
     c->pf_smem = (size_t)(2 * ld8 * ld8 + 2 * ld8) * 8;
     c->pf_grid = max_live;
     if (pref_on && c->pf_smem > 200 * 1024)
@@ -1758,6 +1893,7 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
       q.st = c->d_st;
       q.pref = c->d_pref;
       q.pref_stride = c->pref_stride;
+      q.max_rank = std::max(c->narrow_rank, 1);
       up[n].pref = pref_on ? c->d_pref : nullptr;
       up[n].pref_stride = c->pref_stride;
     }
@@ -2354,9 +2490,11 @@ int cals_b200_clear_models(cals_b200_ctx *c) {
 
 // validation shared by the two enqueue entry points; on success fills `hm` (home_col = first free staging column)
 static int check_model(cals_b200_ctx *c, uint64_t rank, const double *const *host_factors, int jk_mode, int64_t jk_fiber,
-                       int home_col, HostModel *hm) {
+                       int home_col, int id, HostModel *hm) {
   if (rank < 1 || rank > 4096)
     return fail(c, "rank %llu out of range", (unsigned long long)rank);
+  if (check_nnls_rank(c, id, (int)rank))
+    return 1;
   const Geom &geo = c->geo;
   if (jk_mode >= geo.n_modes)
     return fail(c, "jk_mode %d out of range", jk_mode);
@@ -2403,7 +2541,7 @@ int cals_b200_enqueue_model(cals_b200_ctx *c, uint64_t rank, const double *const
   if (!c->have_tensor)
     return fail(c, "set the tensor before enqueueing models");
   HostModel hm;
-  if (check_model(c, rank, host_factors, jk_mode, jk_fiber, c->queued_cols, &hm))
+  if (check_model(c, rank, host_factors, jk_mode, jk_fiber, c->queued_cols, (int)c->hmodels.size(), &hm))
     return 1;
   for (int n = 0; n < c->geo.n_modes; n++)
     if (reserve_input_staging(c, n, (size_t)c->queued_cols + rank, true))
@@ -2432,7 +2570,7 @@ int cals_b200_enqueue_models(cals_b200_ctx *c, uint64_t n_models, const uint64_t
     rows_sum += (size_t)c->geo.dims[n];
   for (uint64_t m = 0; m < n_models; m++) {
     if (check_model(c, ranks[m], host_factors + m * N, jk_modes ? jk_modes[m] : -1, jk_fibers ? jk_fibers[m] : 0, col,
-                    &fresh[m]))
+                    (int)(c->hmodels.size() + m), &fresh[m]))
       return 1;
     col += (int)ranks[m];
   }

@@ -242,15 +242,15 @@ __global__ void __launch_bounds__(256) ls_explicit_error_kernel(const LsParams p
   double acc = 0.0;
   for (long long o = o0; o < o1; o++) {
     __syncthreads();
-    if (tid < R) { // product of the slower modes' trial factors for component tid
+    for (int r = tid; r < R; r += blockDim.x) { // product of the slower modes' trial factors for component r
       long long rem = o;
       double v = 1.0;
       for (int n = 1; n < N; n++) {
         const int idx = (int)(rem % p.geo.dims[n]);
         rem /= p.geo.dims[n];
-        v *= p.prev[n][(size_t)(md.home_col + tid) * p.geo.ldF[n] + idx];
+        v *= p.prev[n][(size_t)(md.home_col + r) * p.geo.ldF[n] + idx];
       }
-      w[tid] = v;
+      w[r] = v;
     }
     __syncthreads();
     const double *x = p.X + o * (long long)p.ldX0;

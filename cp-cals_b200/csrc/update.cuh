@@ -71,6 +71,7 @@ struct PrefactorParams {
   const SchedState *st;
   double *pref;
   long long pref_stride;
+  int max_rank; // largest narrow rank: wide models (wide.cuh) are skipped
 };
 #define CALS_PROF(slot)                                                                                                \
   do {                                                                                                                 \
@@ -574,6 +575,8 @@ __global__ void __launch_bounds__(PREFACTOR_THREADS) prefactor_kernel(const Pref
   if ((int)blockIdx.x >= n_live)
     return;
   const ModelDesc &md = p.models[m];
+  if (md.rank > p.max_rank) // a wide model: wide.cuh
+    return;
   const int R = md.rank, n = p.mode, N = p.n_modes;
   const int LD = (R + 7) & ~7;
   const int tid = threadIdx.x, nthr = blockDim.x;
@@ -627,6 +630,8 @@ model_update_kernel(const UpdateParams p) {
   if ((int)blockIdx.x >= n_live)
     return;
   ModelDesc &md = p.models[m];
+  if (md.rank > p.max_rank) // a wide model: updated by the kernels of wide.cuh
+    return;
   const int R = md.rank, col = md.col, cur = st->cur;
   const int rows = p.rows, ld = p.ld, n = p.mode, N = p.n_modes;
   const int tid = threadIdx.x, nthr = blockDim.x;
