@@ -7,6 +7,8 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
+#include <mutex>
 #include <string>
 #include <thread>
 #include <vector>
@@ -185,8 +187,6 @@ struct cals_b200_ctx {
   std::vector<cudaEvent_t> ev_pool;
   bool dmma_attr_done[16] = {};
   bool pair_attr_done[32] = {}; // [WM]: main instance, [8 + WM]: narrow instance
-  size_t update_attr_smem = 0;
-  size_t leaf_slow_attr = 0;
   // prefactor_kernel (update.cuh) runs on a forked branch: second stream, fork / join events per mode, scratch
   cudaStream_t stream2 = nullptr;
   cudaEvent_t ev_fork[CALS_MAX_MODES] = {}, ev_join[CALS_MAX_MODES] = {};
@@ -197,7 +197,6 @@ struct cals_b200_ctx {
   int wide_slots = 0, wide_ldw = 0, wide_y_rows = 0;
   bool wide_attr_done = false;
   long long pref_stride = 0;
-  size_t prefactor_attr_smem = 0;
   PrefactorParams pf[CALS_MAX_MODES];
   size_t pf_smem = 0;
   int pf_grid = 0;
@@ -291,6 +290,23 @@ cudaError_t launch_chain(cals_b200_ctx *c, void (*kern)(KArgs...), dim3 grid, di
   cfg.attrs = attr;
   cfg.numAttrs = c->pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, KArgs(std::forward<Args>(args))...);
+}
+
+// The dynamic shared-memory limit that cudaFuncSetAttribute sets belongs to the kernel in this process (one per device),
+// not to a context: every context launches the same kernel.  So a limit that follows the problem size (update kernel,
+// TMA-fed leaf, prefactor kernel) only ever grows, to the largest size any context has asked for on that device.  A
+// per-context record of the last value set let a second context with a smaller problem lower the limit below what the
+// first one still launched with, and the first one's next launch failed ("invalid argument").
+int raise_smem_limit(cals_b200_ctx *c, const void *kern, size_t bytes) {
+  static std::mutex mu;
+  static std::map<std::pair<int, const void *>, size_t> limit;
+  std::lock_guard<std::mutex> lock(mu);
+  size_t &cur = limit[{c->device, kern}];
+  if (bytes > cur) {
+    CU_TRY(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    cur = bytes;
+  }
+  return 0;
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -747,13 +763,9 @@ int alloc_buffers(cals_b200_ctx *c, Buffers &b, int cols, bool with_home_cols, i
       if (build_node_slots(c, b))
         return 1;
     }
-    for (int k = 0; k < b.n_nodes; k++) { // dynamic shared memory of the TMA-fed leaf kernel (ring of stages)
-      const size_t ss = leaf_slow_smem(b.node[k].pg.E2);
-      if (ss > c->leaf_slow_attr) {
-        CU_TRY(c, cudaFuncSetAttribute(pair_leaf_slow_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss));
-        c->leaf_slow_attr = ss;
-      }
-    }
+    for (int k = 0; k < b.n_nodes; k++) // dynamic shared memory of the TMA-fed leaf kernel (ring of stages)
+      if (raise_smem_limit(c, (const void *)pair_leaf_slow_tma_kernel, leaf_slow_smem(b.node[k].pg.E2)))
+        return 1;
   }
 
   size_t tiles = 0, tile_elems = 0;
@@ -1598,11 +1610,9 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
     size_t mx = 0;
     for (int n = 0; n < N; n++)
       mx = std::max(mx, up_smem[n]);
-    if (mx > c->update_attr_smem) {
-      CU_TRY(c, cudaFuncSetAttribute(model_update_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
-      CU_TRY(c, cudaFuncSetAttribute(model_update_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mx));
-      c->update_attr_smem = mx;
-    }
+    if (raise_smem_limit(c, (const void *)model_update_kernel<false>, mx) ||
+        raise_smem_limit(c, (const void *)model_update_kernel<true>, mx))
+      return 1;
   }
 
   // slab mode over several GPUs: every MTTKRP is followed by the peer-memory exchange (comm.cuh)
@@ -1879,10 +1889,8 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
     c->pf_grid = max_live;
     if (pref_on && c->pf_smem > 200 * 1024)
       pref_on = false;
-    if (pref_on && c->pf_smem > c->prefactor_attr_smem) {
-      CU_TRY(c, cudaFuncSetAttribute(prefactor_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->pf_smem));
-      c->prefactor_attr_smem = c->pf_smem;
-    }
+    if (pref_on && raise_smem_limit(c, (const void *)prefactor_kernel, c->pf_smem))
+      return 1;
     for (int n = 0; n < N; n++) {
       PrefactorParams &q = c->pf[n];
       q.mode = n;
