@@ -37,7 +37,7 @@ ABI_SYMBOLS = [
     "cals_b200_comm_alloc", "cals_b200_comm_local_block", "cals_b200_comm_connect", "cals_b200_set_tensor_slab",
     "cals_b200_set_tensor_norm", "cals_b200_comm_disconnect", "cals_b200_set_model_active_set",
     "cals_b200_fetch_model_active_set", "cals_b200_set_line_search", "cals_b200_line_search_counts",
-    "cals_b200_enqueue_models", "cals_b200_set_pair_node", "cals_b200_khatri_rao",
+    "cals_b200_enqueue_models", "cals_b200_set_pair_node", "cals_b200_khatri_rao", "cals_b200_core_consistency",
 ]
 
 
@@ -114,6 +114,7 @@ def lib():
     L.cals_b200_line_search_counts.argtypes = [vp, C.POINTER(u64), C.POINTER(u64)]
     L.cals_b200_set_model_active_set.argtypes = [vp, i, C.POINTER(vp)]
     L.cals_b200_fetch_model_active_set.argtypes = [vp, i, C.POINTER(vp)]
+    L.cals_b200_core_consistency.argtypes = [vp, vp, vp]
     _lib = L
     return L
 
@@ -449,6 +450,17 @@ class Engine:
         self._ck(self._L.cals_b200_fetch_all(self._ctx, fptr, lptr, stats))
         return [(fs[m], lams[m], stats[m]) for m in range(M)]
 
+    def core_consistency(self):
+        """Core consistency (CORCONDIA) of every queued model: (cc, status), one entry per model in queue order.  After
+        run / rerun it scores the fitted models, before any run the enqueued factors with lambda = 1.  status 0 =
+        computed, 1 = rank above the limit (96 for 3 modes, 64 for 4), 2 = a Gram matrix A_n^T A_n is not positive
+        definite; cc is NaN unless status is 0."""
+        M = len(getattr(self, "_ranks", []))
+        cc = np.empty(M)
+        status = np.empty(M, dtype=np.int32)
+        self._ck(self._L.cals_b200_core_consistency(self._ctx, cc.ctypes.data, status.ctypes.data))
+        return cc, status
+
     # -- hooks ---------------------------------------------------------------------------------------------------------------
     def mttkrp(self, factors: Sequence[np.ndarray], mode: int, variant: int = MTTKRP_DMMA, repeats: int = 1):
         """G = X_(mode) * KRP(factors except mode) over the concatenated columns.  Returns (G, ms_per_launch)."""
@@ -543,6 +555,30 @@ def cp_cals(X: np.ndarray, ktensors: Sequence[Ktensor], params: CalsParams, *, e
                           mttkrp_launches=rep.mttkrp_launches, kernel_launches=rep.kernel_launches,
                           ls_performed=lsp, ls_failed=lsf, pair_node=bool(rep.tree), tensor_flops=rep.tensor_flops,
                           sweep_period=rep.sweep_period)
+    finally:
+        if own:
+            eng.close()
+
+
+def core_consistency(X: Optional[np.ndarray], ktensors: Sequence[Ktensor], engine: Optional[Engine] = None,
+                     device: int = 0) -> np.ndarray:
+    """Core consistency (Bro & Kiers 2003) of every Ktensor against X, on the device: lambda (when set) is folded into
+    mode 0, jackknife flags are kept (the model leaves out its row of mode 0).  Returns one value per model, NaN for a
+    model whose rank is above the limit or whose factors are rank-deficient (Engine.core_consistency has the status)."""
+    own = engine is None
+    eng = engine or Engine(device)
+    try:
+        if own or eng.modes is None or X is not None:
+            eng.set_tensor(X)
+        eng.clear_models()
+        models = []
+        for kt in ktensors:
+            fs = list(kt.factors)
+            if kt.lam is not None:
+                fs[0] = np.asfortranarray(fs[0] * np.asarray(kt.lam)[None, :])
+            models.append(fs)
+        eng.enqueue_many(models, [(kt.jk_mode, kt.jk_fiber) for kt in ktensors])
+        return eng.core_consistency()[0]
     finally:
         if own:
             eng.close()

@@ -7,6 +7,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <map>
 #include <mutex>
 #include <string>
@@ -19,6 +20,7 @@
 #include "../../include/cals_b200.h"
 #include "comm.cuh"
 #include "common.cuh"
+#include "corcon.cuh"
 #include "ls.cuh"
 #include "mttkrp.cuh"
 #include "pairnode.cuh"
@@ -125,6 +127,7 @@ struct cals_b200_ctx {
   long long gram_doubles = 0;
   bool uploaded = false;
   bool results_fresh = false;
+  bool fitted = false; // the home matrices and d_lambda hold the fitted models of the current queue (run / rerun)
 
   // run-time device state
   Buffers bufs;
@@ -201,6 +204,20 @@ struct cals_b200_ctx {
   size_t pf_smem = 0;
   int pf_grid = 0;
   int fork_mode = -1; // mode whose prefactor branch the next launch_dmma forks between its two kernels (-1: none)
+
+  // core consistency (corcon.cuh): the call's own workspace, kept from call to call and grown when a call needs more;
+  // it never shares memory with the run
+  struct CorconWs {
+    double *F[CALS_MAX_MODES] = {}; // the queue's factors when no fitted models are resident
+    double *P[CALS_MAX_MODES] = {};
+    double *T = nullptr, *chain[2] = {};
+    void *tables = nullptr;
+    SchedState *st = nullptr;
+    double *cc = nullptr;
+    int *status = nullptr, *fail = nullptr;
+    size_t cap_F[CALS_MAX_MODES] = {}, cap_P[CALS_MAX_MODES] = {}, cap_T = 0, cap_chain = 0, cap_tables = 0;
+    size_t cap_st = 0, cap_models = 0;
+  } cc_ws;
 };
 
 namespace {
@@ -1050,6 +1067,7 @@ void release_run(cals_b200_ctx *c) {
     c->ls_prev[n] = c->ls_backup[n] = nullptr;
   c->ls_prev_lambda = c->ls_backup_lambda = c->ls_partial = nullptr;
   c->uploaded = false;
+  c->fitted = false;
   c->run_sig.clear();
 }
 
@@ -1074,8 +1092,26 @@ void release_comm(cals_b200_ctx *c) {
   c->comm_world = 1;
 }
 
+void release_corcon(cals_b200_ctx *c) {
+  auto &w = c->cc_ws;
+  for (int n = 0; n < CALS_MAX_MODES; n++) {
+    cudaFree(w.F[n]);
+    cudaFree(w.P[n]);
+  }
+  cudaFree(w.T);
+  cudaFree(w.chain[0]);
+  cudaFree(w.chain[1]);
+  cudaFree(w.tables);
+  cudaFree(w.st);
+  cudaFree(w.cc);
+  cudaFree(w.status);
+  cudaFree(w.fail);
+  w = cals_b200_ctx::CorconWs();
+}
+
 void release_tensor(cals_b200_ctx *c) {
   release_run(c);
+  release_corcon(c);
   if (c->Xt && c->Xt != c->Xp)
     cudaFree(c->Xt);
   if (c->Xp)
@@ -1278,6 +1314,7 @@ int check_nnls_rank(cals_b200_ctx *c, int model, int rank) {
 int prepare_run(cals_b200_ctx *c) {
   if (!c->have_tensor)
     return fail(c, "no tensor set");
+  c->fitted = false; // the home matrices are overwritten with the initial factors below
   if (c->hmodels.empty())
     return fail(c, "model queue is empty");
   const Geom &geo = c->geo;
@@ -2116,6 +2153,7 @@ int run_loop(cals_b200_ctx *c, cals_b200_report *rep, bool restore_home) {
     }
   }
   c->results_fresh = false;
+  c->fitted = true;
   return 0;
 }
 
@@ -2158,6 +2196,306 @@ void copy_model_out(cals_b200_ctx *c, int m, double *const *factors_out, double 
     stats->old_fit = d.old_fit;
     stats->chol_info = d.chol_info;
   }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Core consistency of every queued model (corcon.cuh).  Models go in queue order, in batches of whole models; a batch
+// holds at most buffer_cols columns, and its T and each of its two chain buffers stay within CC_BATCH_CAP_BYTES (a
+// single model may exceed that on its own).
+constexpr size_t CC_BATCH_CAP_BYTES = (size_t)2 << 30;
+constexpr size_t CC_HEADROOM_BYTES = (size_t)2 << 30; // device memory left free, as for the pair node's T
+
+template <typename T> int cc_grow(cals_b200_ctx *c, T **p, size_t *cap, size_t n) {
+  if (*p && *cap >= n)
+    return 0;
+  cudaFree(*p);
+  *p = nullptr;
+  *cap = 0;
+  CU_TRY(c, cudaMalloc((void **)p, std::max<size_t>(n, 1) * sizeof(T)));
+  *cap = n;
+  return 0;
+}
+
+template <int WM>
+int launch_cc_pair_gemm(cals_b200_ctx *c, const PairMaps &maps, const PairGeom &pg, const SchedState *st, double *T) {
+  auto kern = pair_gemm_kernel<WM, WN_FIXED>;
+  constexpr int smem = PairCfg<WM, WN_FIXED>::SMEM_BYTES;
+  if (raise_smem_limit(c, (const void *)kern, smem))
+    return 1;
+  kern<<<c->sm_count, MTTKRP_THREADS, smem, c->stream>>>(maps, pg, st, T, nullptr);
+  CU_TRY(c, cudaGetLastError());
+  return 0;
+}
+
+int core_consistency(cals_b200_ctx *c, double *cc_out, int32_t *status_out) {
+  if (!c->have_tensor)
+    return fail(c, "no tensor set");
+  const Geom &geo = c->geo;
+  const int N = geo.n_modes, M = (int)c->hmodels.size();
+  if (N > 4)
+    return fail(c, "core consistency supports tensors of 3 and 4 modes, this one has %d", N);
+  if (c->slice_mode >= 0)
+    return fail(c, "core consistency needs the whole tensor on one device; this context holds a slab of mode %d",
+                c->slice_mode);
+  if (M == 0)
+    return 0;
+  cudaStream_t s = c->stream;
+  auto &w = c->cc_ws;
+  const int *dims = geo.dims;
+
+  // statuses known before any computation: 1 = rank above the limit, 2 = rank above an extent (A_n^T A_n is singular)
+  const int limit = N == 3 ? narrow_rank_bound(false) : CC_MAX_RANK_4;
+  std::vector<int32_t> status(M, 0);
+  for (int m = 0; m < M; m++) {
+    const int R = c->hmodels[m].rank;
+    if (R > limit)
+      status[m] = 1;
+    else
+      for (int n = 0; n < N; n++)
+        if (R > dims[n])
+          status[m] = 2;
+    if (status[m] == 0 && R > c->buffer_cols)
+      return fail(c, "model %d has rank %d > buffer_size %d", m, R, c->buffer_cols);
+  }
+
+  // batches, and every model's jobs in the contraction steps s = 1 .. N-1 (output of step s: chain[(s - 1) & 1])
+  long long rest = 1; // prod_{n >= 2} I_n
+  for (int n = 2; n < N; n++)
+    rest *= dims[n];
+  const long long ldT = (long long)dims[1] * rest;
+  auto out_size = [&](int R, int step) { // (prod_{n > step} I_n) * R^(step + 1)
+    long long v = 1;
+    for (int n = step + 1; n < N; n++)
+      v *= dims[n];
+    for (int k = 0; k <= step; k++)
+      v *= R;
+    return v;
+  };
+  const long long cap = (long long)(CC_BATCH_CAP_BYTES / 8);
+  std::vector<CcModel> bm;
+  std::vector<int> bstart{0};       // batch b: bm[bstart[b] .. bstart[b + 1])
+  std::vector<int> bcols;
+  std::vector<long long> bchain[2];
+  int cols = 0, max_cols = 0;
+  long long ch[2] = {0, 0}, max_chain[2] = {0, 0};
+  auto close_batch = [&]() {
+    bstart.push_back((int)bm.size());
+    bcols.push_back(cols);
+    max_cols = std::max(max_cols, cols);
+    for (int k = 0; k < 2; k++) {
+      bchain[k].push_back(ch[k]);
+      max_chain[k] = std::max(max_chain[k], ch[k]);
+      ch[k] = 0;
+    }
+    cols = 0;
+  };
+  for (int m = 0; m < M; m++) {
+    if (status[m] != 0)
+      continue;
+    const HostModel &hm = c->hmodels[m];
+    const int R = hm.rank;
+    long long add[2] = {0, 0};
+    for (int st = 1; st < N; st++)
+      add[(st - 1) & 1] = std::max(add[(st - 1) & 1], out_size(R, st));
+    const bool full = cols + R > c->buffer_cols || (long long)(cols + R) * ldT > cap || ch[0] + add[0] > cap ||
+                      ch[1] + add[1] > cap;
+    if (cols > 0 && full)
+      close_batch();
+    bm.push_back(CcModel{m, R, hm.home_col, cols, hm.jk_mode == 0 ? hm.jk_fiber : -1});
+    cols += R;
+    ch[0] += add[0];
+    ch[1] += add[1];
+  }
+  if (cols > 0)
+    close_batch();
+  const int n_batches = (int)bcols.size(), n_bm = (int)bm.size();
+  // jobs[(step - 1) * n_bm + i] for batch model i; offsets and first tiles count from the start of its batch
+  std::vector<CcJob> jobs((size_t)(N - 1) * n_bm);
+  std::vector<long long> tiles((size_t)(N - 1) * n_batches, 0);
+  for (int b = 0; b < n_batches; b++)
+    for (int st = 1; st < N; st++) {
+      long long off = 0, t0 = 0;
+      for (int i = bstart[b]; i < bstart[b + 1]; i++) {
+        CcJob &j = jobs[(size_t)(st - 1) * n_bm + i];
+        const int R = bm[i].rank;
+        j.R = R;
+        j.bcol = bm[i].bcol;
+        j.in_off = st == 1 ? (long long)bm[i].bcol * ldT : jobs[(size_t)(st - 2) * n_bm + i].out_off;
+        j.out_off = off;
+        j.M = out_size(R, st) / R;
+        j.tile0 = t0;
+        off += out_size(R, st);
+        t0 += (j.M + CC_CHAIN_MT - 1) / CC_CHAIN_MT;
+      }
+      tiles[(size_t)(st - 1) * n_batches + b] = t0;
+    }
+
+  // workspace: grown when this call needs more than the last one; 2 GB of device memory stay free
+  const size_t job_bytes = jobs.size() * sizeof(CcJob), table_bytes = job_bytes + bm.size() * sizeof(CcModel);
+  {
+    size_t need = 0;
+    auto more = [&](size_t cap_now, size_t n, size_t elem) { need += cap_now >= n ? 0 : n * elem; };
+    for (int n = 0; n < N; n++) {
+      if (!c->fitted)
+        more(w.cap_F[n], (size_t)geo.ldF[n] * c->queued_cols, 8);
+      more(w.cap_P[n], (size_t)geo.ldF[n] * max_cols, 8);
+    }
+    more(w.cap_T, (size_t)ldT * max_cols, 8);
+    more(w.cap_chain, (size_t)std::max(max_chain[0], max_chain[1]), 16);
+    size_t free_b = 0, total_b = 0;
+    CU_TRY(c, cudaMemGetInfo(&free_b, &total_b));
+    if (need + CC_HEADROOM_BYTES > free_b)
+      return fail(c, "core consistency needs %.1f GB more device memory, %.1f GB are free", need / 1e9, free_b / 1e9);
+  }
+  const double *F[CALS_MAX_MODES] = {};
+  const double *lambda = nullptr;
+  for (int n = 0; n < N; n++) {
+    if (c->fitted) { // after run / rerun: the fitted factors and lambda
+      F[n] = c->bufs.fac.home[n];
+      lambda = c->d_lambda;
+    } else { // the queue as enqueued, lambda = 1 (the pinned staging already has the device layout)
+      const size_t count = (size_t)geo.ldF[n] * c->queued_cols;
+      if (cc_grow(c, &w.F[n], &w.cap_F[n], count))
+        return 1;
+      CU_TRY(c, cudaMemcpyAsync(w.F[n], c->h_in[n], count * 8, cudaMemcpyHostToDevice, s));
+      F[n] = w.F[n];
+    }
+    if (cc_grow(c, &w.P[n], &w.cap_P[n], (size_t)geo.ldF[n] * max_cols))
+      return 1;
+  }
+  if (cc_grow(c, &w.T, &w.cap_T, (size_t)ldT * max_cols))
+    return 1;
+  if (w.cap_chain < (size_t)std::max(max_chain[0], max_chain[1])) {
+    size_t dummy = 0;
+    if (cc_grow(c, &w.chain[0], &w.cap_chain, (size_t)std::max(max_chain[0], max_chain[1])) ||
+        cc_grow(c, &w.chain[1], &dummy, w.cap_chain))
+      return 1;
+  }
+  unsigned char *tab = nullptr;
+  if (cc_grow(c, (unsigned char **)&w.tables, &w.cap_tables, table_bytes) ||
+      cc_grow(c, &w.st, &w.cap_st, (size_t)std::max(n_batches, 1)) || cc_grow(c, &w.cc, &w.cap_models, (size_t)M))
+    return 1;
+  if (w.cap_models > 0) {
+    size_t cs = 0, cf = 0;
+    if (cc_grow(c, &w.status, &cs, w.cap_models) || cc_grow(c, &w.fail, &cf, w.cap_models * N))
+      return 1;
+  }
+  tab = (unsigned char *)w.tables;
+  const CcJob *d_jobs = (const CcJob *)tab;
+  const CcModel *d_bm = (const CcModel *)(tab + job_bytes);
+  if (n_bm > 0) {
+    std::vector<unsigned char> host(table_bytes);
+    memcpy(host.data(), jobs.data(), job_bytes);
+    memcpy(host.data() + job_bytes, bm.data(), bm.size() * sizeof(CcModel));
+    CU_TRY(c, cudaMemcpyAsync(tab, host.data(), table_bytes, cudaMemcpyHostToDevice, s));
+    std::vector<SchedState> sts(n_batches);
+    for (int b = 0; b < n_batches; b++) {
+      sts[b] = SchedState{};
+      sts[b].C = sts[b].C_main = bcols[b];
+    }
+    CU_TRY(c, cudaMemcpyAsync(w.st, sts.data(), sts.size() * sizeof(SchedState), cudaMemcpyHostToDevice, s));
+  }
+
+  int max_dim = 0;
+  for (int n = 0; n < N; n++)
+    max_dim = std::max(max_dim, dims[n]);
+  for (int b = 0; b < n_batches; b++) {
+    const int i0 = bstart[b], nb = bstart[b + 1] - i0, C = bcols[b];
+    // 1. pseudo-inverses
+    CcPinvParams pp{};
+    pp.n_modes = N;
+    for (int n = 0; n < N; n++) {
+      pp.dims[n] = dims[n];
+      pp.ld[n] = geo.ldF[n];
+      pp.F[n] = F[n];
+      pp.P[n] = w.P[n];
+    }
+    pp.lambda = lambda;
+    pp.models = d_bm + i0;
+    pp.fail = w.fail;
+    size_t smem = 0;
+    for (int i = i0; i < i0 + nb; i++)
+      smem = std::max(smem, cc_pinv_smem(bm[i].rank, cc_chunk_rows(bm[i].rank, max_dim) + 4));
+    pp.max_rows = max_dim;
+    if (raise_smem_limit(c, (const void *)corcon_pinv_kernel, smem))
+      return 1;
+    corcon_pinv_kernel<<<dim3(nb, N), CC_THREADS, smem, s>>>(pp);
+    CU_TRY(c, cudaGetLastError());
+    // 2. T = X x_0 P_0 over the batch's columns: pair_gemm_kernel on the 3-D view (I_0, I_1, prod_{n>=2} I_n) of Xp
+    PairMaps maps{};
+    PairGeom pg{};
+    pg.E1 = dims[1];
+    pg.E2 = (int)rest;
+    pg.R = (int)ldT;
+    pg.ldT = ldT;
+    pg.Ip = dims[0];
+    pg.mode_fast = 1;
+    pg.mode_slow = 2;
+    for (int n = 0; n < N; n++)
+      pg.ldF[n] = geo.ldF[n];
+    pg.ld_fast = geo.ldF[1];
+    const int wm = pick_pair_wm(pg.E1, pg.E2, C, c->sm_count);
+    {
+      cuuint64_t dx[3] = {(cuuint64_t)dims[0], (cuuint64_t)dims[1], (cuuint64_t)rest};
+      cuuint64_t sx[2] = {(cuuint64_t)c->ldX0 * 8, (cuuint64_t)c->ldX0 * dims[1] * 8};
+      cuuint32_t bx[3] = {(cuuint32_t)KT, 8, (cuuint32_t)wm};
+      cuuint64_t d2[2] = {(cuuint64_t)dims[0], (cuuint64_t)C};
+      cuuint64_t s2[1] = {(cuuint64_t)geo.ldF[0] * 8};
+      cuuint32_t b2[2] = {(cuuint32_t)KT, (cuuint32_t)TILE_N};
+      if (encode_map(c, &maps.X, c->Xp, 3, dx, sx, bx) || encode_map(c, &maps.B[0], w.P[0], 2, d2, s2, b2))
+        return 1;
+      maps.B[1] = maps.B[0];
+    }
+    const SchedState *st = w.st + b;
+    int rc;
+    switch (wm) {
+    case 4:
+      rc = launch_cc_pair_gemm<4>(c, maps, pg, st, w.T);
+      break;
+    case 5:
+      rc = launch_cc_pair_gemm<5>(c, maps, pg, st, w.T);
+      break;
+    case 6:
+      rc = launch_cc_pair_gemm<6>(c, maps, pg, st, w.T);
+      break;
+    case 7:
+      rc = launch_cc_pair_gemm<7>(c, maps, pg, st, w.T);
+      break;
+    default:
+      rc = launch_cc_pair_gemm<8>(c, maps, pg, st, w.T);
+    }
+    if (rc)
+      return 1;
+    // 3. the per-model chain, one launch per contracted mode
+    for (int stp = 1; stp < N; stp++) {
+      const long long grid = tiles[(size_t)(stp - 1) * n_batches + b];
+      if (grid > 0x7fffffffLL)
+        return fail(c, "core consistency: %lld tiles in one contraction step", grid);
+      const double *in = stp == 1 ? w.T : w.chain[(stp - 2) & 1];
+      corcon_chain_kernel<<<(unsigned)grid, CC_THREADS, 0, s>>>(d_jobs + (size_t)(stp - 1) * n_bm + i0, nb, dims[stp],
+                                                                 in, w.P[stp], geo.ldF[stp], w.chain[(stp - 1) & 1]);
+      CU_TRY(c, cudaGetLastError());
+    }
+    corcon_final_kernel<<<nb, CC_FINAL_THREADS, 0, s>>>(d_bm + i0, d_jobs + (size_t)(N - 2) * n_bm + i0, N,
+                                                        w.chain[(N - 2) & 1], w.fail, w.cc, w.status);
+    CU_TRY(c, cudaGetLastError());
+  }
+
+  std::vector<double> dcc(M);
+  std::vector<int32_t> dst(M);
+  if (n_bm > 0) {
+    CU_TRY(c, cudaMemcpyAsync(dcc.data(), w.cc, (size_t)M * 8, cudaMemcpyDeviceToHost, s));
+    CU_TRY(c, cudaMemcpyAsync(dst.data(), w.status, (size_t)M * 4, cudaMemcpyDeviceToHost, s));
+  }
+  CU_TRY(c, cudaStreamSynchronize(s));
+  for (const CcModel &x : bm)
+    status[x.model] = dst[x.model];
+  for (int m = 0; m < M; m++) {
+    cc_out[m] = status[m] == 0 ? dcc[m] : std::numeric_limits<double>::quiet_NaN();
+    if (status_out)
+      status_out[m] = status[m];
+  }
+  return 0;
 }
 
 } // namespace
@@ -2492,6 +2830,7 @@ int cals_b200_clear_models(cals_b200_ctx *c) {
   c->h_active.clear();
   c->queued_cols = 0;
   c->uploaded = false;
+  c->fitted = false;
   c->results_fresh = false;
   return 0;
 }
@@ -2558,6 +2897,7 @@ int cals_b200_enqueue_model(cals_b200_ctx *c, uint64_t rank, const double *const
   c->queued_cols += (int)rank;
   c->hmodels.push_back(hm);
   c->uploaded = false;
+  c->fitted = false;
   if (model_id)
     *model_id = (int)c->hmodels.size() - 1;
   return 0;
@@ -2592,6 +2932,7 @@ int cals_b200_enqueue_models(cals_b200_ctx *c, uint64_t n_models, const uint64_t
   c->queued_cols = col;
   c->hmodels.insert(c->hmodels.end(), fresh.begin(), fresh.end());
   c->uploaded = false;
+  c->fitted = false;
   return 0;
 }
 
@@ -2883,6 +3224,13 @@ int cals_b200_device_info(cals_b200_ctx *c, int *sm_count, size_t *free_bytes, s
   if (total_bytes)
     *total_bytes = t;
   return 0;
+}
+
+int cals_b200_core_consistency(cals_b200_ctx *c, double *cc_out, int32_t *status_out) {
+  if (!c || !cc_out)
+    return fail(c, "null argument");
+  cudaSetDevice(c->device);
+  return core_consistency(c, cc_out, status_out);
 }
 
 } // extern "C"

@@ -558,6 +558,54 @@ JKReport jk_cp_cals(const Tensor &X, vector<Ktensor> &kt_vector, CalsParams &cal
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
+std::vector<double> core_consistency(const Tensor &X, const std::vector<Ktensor> &models, int device) {
+  detail::EngineHandle &e = detail::engine_for_device(device);
+  std::lock_guard<std::mutex> lk(e.mu);
+  const size_t M = models.size();
+  std::vector<double> cc(M);
+  if (M == 0)
+    return cc;
+  detail::upload_tensor(e, X, false);
+  const dim_t N = X.get_n_modes();
+  // lambda folded into mode 0 (the engine takes lambda = 1 for enqueued models)
+  std::vector<std::vector<double>> first(M);
+  std::vector<const double *> in(M * N);
+  std::vector<uint64_t> ranks(M);
+  std::vector<int> jk_modes(M);
+  std::vector<int64_t> jk_fibers(M);
+  for (size_t m = 0; m < M; m++) {
+    const Ktensor &kt = models[m];
+    if (kt.get_n_modes() != N)
+      throw B200Error("core_consistency: a Ktensor has a different number of modes than the tensor");
+    const dim_t R = kt.get_components();
+    for (dim_t n = 0; n < N; n++) {
+      if (kt.get_factor(n).get_rows() != X.get_modes()[n])
+        throw B200Error("core_consistency: a Ktensor factor does not match the tensor extents");
+      in[m * N + n] = kt.get_factor(n).get_data();
+    }
+    const Matrix &F0 = kt.get_factor(0);
+    const dim_t rows = F0.get_rows();
+    const std::vector<double> &lam = kt.get_lambda();
+    first[m].assign(F0.get_data(), F0.get_data() + rows * R);
+    for (dim_t j = 0; j < R && j < lam.size(); j++)
+      for (dim_t i = 0; i < rows; i++)
+        first[m][i + j * rows] *= lam[j];
+    in[m * N] = first[m].data();
+    ranks[m] = R;
+    jk_modes[m] = kt.is_jk() ? (int)kt.get_jk_mode() : -1;
+    jk_fibers[m] = kt.is_jk() ? (int64_t)kt.get_jk_fiber() : 0;
+  }
+  // the pooled context keeps the buffer size of its last run; batches of the default size (cp_cals configures again)
+  const dim_t buffer = std::max<dim_t>(4200, *std::max_element(ranks.begin(), ranks.end()));
+  detail::check(e, cals_b200_configure(e.ctx, buffer, 200, 1e-7, 0u), "cals_b200_configure");
+  detail::check(e, cals_b200_clear_models(e.ctx), "cals_b200_clear_models");
+  detail::check(e, cals_b200_enqueue_models(e.ctx, M, ranks.data(), in.data(), jk_modes.data(), jk_fibers.data()),
+                "cals_b200_enqueue_models");
+  detail::check(e, cals_b200_core_consistency(e.ctx, cc.data(), nullptr), "cals_b200_core_consistency");
+  return cc;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
 void CalsParams::print() const {
   using std::cout;
   using std::endl;

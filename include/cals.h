@@ -117,5 +117,11 @@ CalsReport cp_cals(const Tensor &X, KtensorQueue &kt_queue, CalsParams &cals_par
 
 JKReport jk_cp_cals(const Tensor &X, vector<Ktensor> &kt_vector, CalsParams &cals_params);
 
+// Extension (no reference counterpart): the core consistency diagnostic (CORCONDIA, Bro & Kiers, J. Chemometrics 17
+// (2003) 274-286) of every model against X, computed on one device.  Lambda is folded into mode 0; a jackknife model
+// leaves out its row of mode 0.  3- and 4-mode tensors; NaN for a model of rank above the limit (96 for 3 modes, 64 for
+// 4) or with a rank-deficient factor.
+std::vector<double> core_consistency(const Tensor &X, const std::vector<Ktensor> &models, int device = 0);
+
 } // namespace cals
 #endif

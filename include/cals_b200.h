@@ -156,6 +156,18 @@ int cals_b200_fetch_model(cals_b200_ctx *ctx, int model_id, double *const *facto
 int cals_b200_fetch_all(cals_b200_ctx *ctx, double *const *factors_out, double *const *lambda_out,
                         cals_b200_model_stats *stats);
 
+/* ---- core consistency (CORCONDIA, Bro & Kiers, J. Chemometrics 17 (2003) 274-286; extension, no reference
+ * counterpart) ---------------------------------------------------------------------------------------------------- */
+/* The core consistency diagnostic of every queued model, computed on the device: CC = 100 (1 - sum (G - I)^2 / R) with G
+ * the least-squares Tucker core of X for the model's factors (A_0 = F_0 diag(lambda), A_n = F_n) and I the superdiagonal
+ * identity.  After cals_b200_run / cals_b200_rerun the fitted factors and lambda are used; before any run (or after
+ * the queue changed) the enqueued factors with lambda = 1.  A jackknife model leaves out its row of mode 0.
+ * cc_out and status_out (may be NULL) get one entry per queued model, in model-id order; status 0 = computed,
+ * 1 = rank above the limit (96 for 3 modes, 64 for 4), 2 = some A_n^T A_n is not numerically positive definite (rank
+ * above an extent, equal columns, lambda = 0); cc is NaN unless the status is 0.  Tensors of 3 and 4 modes held whole by
+ * this device only.  Nothing that a later fetch, run or rerun returns changes. */
+int cals_b200_core_consistency(cals_b200_ctx *ctx, double *cc_out, int32_t *status_out);
+
 /* ---- NNLS active sets (Ktensor::active_set, reference include/ktensor.h:36; they persist across calls there) ---- */
 /* active[n] / active_out[n] -> I_n x rank bytes, row-major (byte [row * rank + col]); 1 = the entry is constrained
  * to zero.  Models start with every constraint active unless set here after enqueueing; fetch after a run. */
